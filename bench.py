@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- stage-1 input GB/s on B200 (BASELINE.json metric), one JSON line on rank 0.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (synthetic, deterministic; mojo_simdjson_b200/synth/gen.c):
   N = 1 : BASELINE.json configs[2] -- ONE 1 GiB JSON document (array of minified twitter-like statuses).
@@ -25,6 +25,12 @@ flushes it explicitly.
 --impl reference times the CPU restatement of the reference's stage 1 (oracle/, kind "port": the reference is Mojo
 and cannot be built in this image) on the host cores, on a bounded sample of the same workload (its size is printed in
 `config`), and reports the AVX-512 / pclmulqdq "cpu_simd" stage 1 of the same specification beside it.
+
+--dump-outputs DIR writes, after the timed steps, what the timed path computed in its last step: stage1_result.npy (the
+verdict rows) and a fixed, seeded sample of the index stream with its positions (structural_indexes.npy,
+structural_index_positions.npy), all float64, 32 MiB at most.  The inputs are generated from fixed seeds, so two builds run
+with the same arguments can be compared file for file.  (--impl reference sizes its sample from a timing probe: its dumps
+compare where `config.reference_sample_bytes_per_step` agrees.)
 """
 from __future__ import annotations
 
@@ -144,7 +150,13 @@ def parse_args():
     ap.add_argument("--no-utf8", action="store_true", help="skip UTF-8 validation (the reference validates nothing)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample-bytes", type=int, default=GIB)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path computed in its last step to DIR/<name>.npy "
+                         "(float64; the index stream as a fixed, seeded sample): compares two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -202,6 +214,75 @@ def workload_config(n_gpus: int, config: str, size: int, total: int = 0, seg_byt
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: the last timed step's results, so that two builds can be compared output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_ENTRIES = 2 << 20     # index entries sampled in all: values + positions in float64 = 32 MiB, under the 64 MiB limit
+DUMP_SEED = 0x5EED0D06
+
+
+def sample_positions(m: int, k: int):
+    """Which entries of an m-entry index stream are dumped: all of them when m <= k; otherwise the first and the last k/4
+    (the document's start, its end and the 3-entry trailer) and one seeded position in each of k/2 equal strata in
+    between.  Depends on m alone, so two builds that agree on the count dump the same positions."""
+    import numpy as np
+
+    if m <= k:
+        return np.arange(m, dtype=np.int64)
+    edge = k // 4
+    c, span = k - 2 * edge, m - 2 * edge
+    lo = edge + np.arange(c, dtype=np.int64) * span // c
+    hi = edge + (np.arange(c, dtype=np.int64) + 1) * span // c
+    mid = lo + (np.random.default_rng(DUMP_SEED).random(c) * (hi - lo)).astype(np.int64)
+    return np.concatenate([np.arange(edge, dtype=np.int64), mid, np.arange(m - edge, m, dtype=np.int64)])
+
+
+def index_stream_sample(streams, k: int) -> dict:
+    """A sample of the index streams of the last step (uint32 / int32 numpy arrays or device tensors, read as one
+    concatenated stream) and the positions sampled."""
+    import numpy as np
+    import torch
+
+    starts = np.cumsum([0] + [len(s) for s in streams])
+    pos = sample_positions(int(starts[-1]), k)
+    piece = np.searchsorted(starts, pos, side="right") - 1
+    vals = []
+    for i, s in enumerate(streams):
+        p = pos[piece == i] - starts[i]
+        v = s[p] if isinstance(s, np.ndarray) else s[torch.from_numpy(p).to(s.device)].cpu().numpy()
+        vals.append(v.astype(np.int64) & 0xFFFFFFFF)
+    return {"structural_indexes": np.concatenate(vals), "structural_index_positions": pos}
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    """out_dir/<name>.npy in float64 for every array (indexes, counts and error codes are below 2^53: exact)."""
+    import numpy as np
+
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the 64 MiB limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def dump_last_step(args, result, streams, suffix: str = "", k: int = DUMP_ENTRIES) -> None:
+    """result: the last step's verdicts, one row per document: (error, n or -1, entries written, UTF-8 verdict), or the
+    batch driver's {error, n} rows."""
+    if args.dump_outputs:
+        arrays = {"stage1_result": result, **index_stream_sample(streams, k)}
+        write_outputs(args.dump_outputs, {name + suffix: a for name, a in arrays.items()})
+
+
+def dump_last_device_step(args, ctx, d_out) -> None:
+    """The last call enqueued on ctx (device-resident path): its verdict, and its index stream in d_out."""
+    if args.dump_outputs:
+        r = ctx.finish()
+        n = -1 if r.n is None else r.n
+        dump_last_step(args, [(r.error, n, r.n_written, r.utf8_error)], [d_out[: n + 3 if n >= 0 else r.n_written]])
+
+
+# ------------------------------------------------------------------------------------------------
 # CPU arm (oracle port of the reference) -- the only place besides tests/smoke that runs oracle/
 # ------------------------------------------------------------------------------------------------
 def _run_pieces(fn, threads: int, repeats: int):
@@ -219,10 +300,11 @@ def _run_pieces(fn, threads: int, repeats: int):
     return best
 
 
-def cpu_stage1_gbs(sample, threads: int, repeats: int = 1, impl: str = "port"):
+def cpu_stage1_gbs(sample, threads: int, repeats: int = 1, impl: str = "port", last: list | None = None):
     """Times the CPU stage 1 on `sample`, split into `threads` independent pieces run concurrently (ctypes releases the
     GIL).  impl "port": oracle_stage1_ref, the block-for-block restatement of the reference incl. its 64-iteration
-    prefix_xor; "simd": oracle/stage1_simd.c, AVX-512 / AVX2 + pclmulqdq stage 1 of the same specification."""
+    prefix_xor; "simd": oracle/stage1_simd.c, AVX-512 / AVX2 + pclmulqdq stage 1 of the same specification.
+    last (port only): receives, per piece, ((error, n or -1, entries written, UTF-8 verdict), index stream) of the last pass."""
     import numpy as np
 
     from oracle import oracle
@@ -231,12 +313,15 @@ def cpu_stage1_gbs(sample, threads: int, repeats: int = 1, impl: str = "port"):
     piece = (n_bytes + threads - 1) // threads
     parts = [sample[i * piece : min(n_bytes, (i + 1) * piece)] for i in range(threads)]
     outs = [np.empty(p.size // 3 + 64, dtype=np.uint32) for p in parts]
+    results = [None] * threads
     if impl == "port":
         L = oracle.lib(native=True)
 
         def work(i):
-            n, nw, u8 = C.c_uint32(0), C.c_uint64(0), C.c_int32(0)
-            L.oracle_stage1_ref(parts[i].ctypes.data, parts[i].size, outs[i].ctypes.data, outs[i].size, C.byref(n), C.byref(nw), C.byref(u8), 0)
+            n, nw, u8 = C.c_uint32(0xFFFFFFFF), C.c_uint64(0), C.c_int32(0)
+            err = L.oracle_stage1_ref(parts[i].ctypes.data, parts[i].size, outs[i].ctypes.data, outs[i].size, C.byref(n), C.byref(nw),
+                                      C.byref(u8), 0)
+            results[i] = (err, -1 if n.value == 0xFFFFFFFF else n.value, nw.value, u8.value)
     else:
         L = oracle.simd_lib()
 
@@ -244,6 +329,9 @@ def cpu_stage1_gbs(sample, threads: int, repeats: int = 1, impl: str = "port"):
             n, nw, u8 = C.c_uint32(0), C.c_uint64(0), C.c_int32(0)
             L.simd_stage1(parts[i].ctypes.data, parts[i].size, outs[i].ctypes.data, outs[i].size, C.byref(n), C.byref(nw), C.byref(u8), 0, 0)
     best = _run_pieces(work, threads, repeats)
+    if last is not None:
+        # the stream is n + 3 entries (the trailer) when n was assigned, else the entries written before the early return
+        last[:] = [(r, outs[i][: r[1] + 3 if r[1] >= 0 else r[2]]) for i, r in enumerate(results)]
     return n_bytes / best / 1e9, best
 
 
@@ -323,9 +411,11 @@ def run_reference(args):
     for _ in range(args.warmup):
         cpu_stage1_gbs(sample, threads)
     t_total = 0.0
+    last = []
     for _ in range(args.steps):
-        _, dt = cpu_stage1_gbs(sample, threads)
+        _, dt = cpu_stage1_gbs(sample, threads, last=last)
         t_total += dt
+    dump_last_step(args, [r for r, _ in last], [s for _, s in last])
     gbs = per_step * args.steps / t_total / 1e9
     sample_desc = (f"{per_step} bytes ({per_step / (1 << 20):.1f} MiB) of the same generator per step, {args.steps} timed steps after "
                    f"{args.warmup} warm-up steps, {threads} thread(s); CPU: {cpu_model()}, {cores} cores")
@@ -412,6 +502,7 @@ def run_small(args, torch, np, dev, local):
     torch.cuda.synchronize()
     cold_us = sorted(1e3 * a.elapsed_time(b) for a, b in cold)
     launches = ctx.launch_count() - launches0
+    dump_last_device_step(args, ctx, d_out)   # the timed figure is the cold launches': their last one
     # (2) back to back (L2 warm), one event pair around K launches
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
@@ -590,10 +681,17 @@ def run_ours(args):
         step()
     host_enqueue_ms = (time.perf_counter() - t_host0) * 1e3 / args.steps   # CPU time to issue one pass (diagnostic)
     if driver is not None:
-        driver.finish()   # the last verdict exchanges belong to the timed region (the host waits for them, then records)
+        _, last_rows = driver.finish()   # the last verdict exchanges belong to the timed region (the host waits for them, then records)
     ev1.record(stream)
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if n_gpus == 1:
+        dump_last_device_step(args, ctx, d_out)
+    elif args.dump_outputs:
+        # this rank's segments; every rank holds the all-gathered {error, n} rows of all of them
+        rows = last_rows[rank, :nseg].tolist()
+        streams = [d_out[idx_offsets[s] : idx_offsets[s] + (n + 3 if e == 0 else 0)] for s, (e, n) in enumerate(rows)]
+        dump_last_step(args, last_rows.reshape(-1, 2), streams, suffix=f"_rank{rank}", k=DUMP_ENTRIES // world)
     if world > 1:
         dist.barrier()
         torch.cuda.synchronize()

@@ -10,6 +10,7 @@ import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 from dataclasses import dataclass
 
 import numpy as np
@@ -32,24 +33,33 @@ def _cpu_signature() -> str:
     return "unknown"
 
 
+def _build_native(src: str) -> str:
+    """The -march=native build goes to a per-user temporary directory, never into the tree: bench.py must run from a
+    read-only checkout, and a build for one CPU must not travel with the tree to another.  The file name carries a digest
+    of the source, the Makefile and the CPU's feature flags, so a different checkout or host never picks up a stale build."""
+    h = hashlib.sha1(_cpu_signature().encode())
+    for p in (src, os.path.join(_HERE, "Makefile")):
+        with open(p, "rb") as f:
+            h.update(f.read())
+    d = os.path.join(tempfile.gettempdir(), f"sjb200-oracle-{os.getuid()}")
+    path = os.path.join(d, f"liboracle_stage1_native-{h.hexdigest()[:16]}.so")
+    if not os.path.exists(path):
+        os.makedirs(d, mode=0o700, exist_ok=True)
+        tmp = f"{path}.{os.getpid()}.tmp"   # concurrent ranks each build their own, then rename atomically
+        subprocess.check_call(["make", "-s", "-C", _HERE, f"NATIVE_OUT={tmp}", tmp])
+        os.replace(tmp, path)
+    return path
+
+
 def build(native: bool = False) -> str:
-    target = "liboracle_stage1_native.so" if native else "liboracle_stage1.so"
-    path = os.path.join(_HERE, target)
     src = os.path.join(_HERE, "stage1_oracle.c")
-    stale = not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(src)
-    sig_path = path + ".cpu"
-    if native and not stale:   # built on another machine (it travels with the repository snapshot)?
-        try:
-            stale = open(sig_path).read().strip() != _cpu_signature()
-        except OSError:
-            stale = True
-    if stale:
+    if native:
+        return _build_native(src)
+    path = os.path.join(_HERE, "liboracle_stage1.so")
+    if not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(src):
         if os.path.exists(path):
             os.remove(path)
-        subprocess.check_call(["make", "-s", "-C", _HERE, target])
-        if native:
-            with open(sig_path, "w") as f:
-                f.write(_cpu_signature())
+        subprocess.check_call(["make", "-s", "-C", _HERE, "liboracle_stage1.so"])
     return path
 
 
