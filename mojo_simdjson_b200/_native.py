@@ -5,8 +5,7 @@ import ctypes as C
 import os
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
-_VARIANT = os.environ.get("SJB200_LIB_VARIANT", "")  # experiment builds only (mojo_simdjson_b200.build.build_variant)
-LIB_PATH = os.path.join(_PKG, f"libsimdjson_b200_{_VARIANT}.so" if _VARIANT else "libsimdjson_b200.so")
+LIB_PATH = os.path.join(_PKG, "libsimdjson_b200.so")
 
 FLAG_VALIDATE_UTF8 = 1
 FLAG_NO_UTF8 = 4

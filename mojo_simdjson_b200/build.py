@@ -37,14 +37,6 @@ def build_cuda(force: bool = False, verbose: bool = False) -> str:
     return LIB
 
 
-def build_variant(name: str, defines: list[str]) -> str:
-    """Experiment builds: libsimdjson_b200_<name>.so with extra -D flags (selected with SJB200_LIB_VARIANT)."""
-    out = os.path.join(PKG, f"libsimdjson_b200_{name}.so")
-    nvcc = os.environ.get("NVCC", "nvcc")
-    subprocess.check_call([nvcc] + NVCC_FLAGS + [f"-D{d}" for d in defines] + ["-o", out, os.path.join(CSRC, "capi.cu")])
-    return out
-
-
 def build_synth(force: bool = False) -> str:
     if force or _stale(SYNTH_LIB, [SYNTH_SRC]):
         subprocess.check_call(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-o", SYNTH_LIB, SYNTH_SRC])

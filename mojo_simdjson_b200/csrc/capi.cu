@@ -13,10 +13,6 @@
 #include "stage1_split.cuh"
 #include "stage1_stream.cuh"
 
-#ifndef SJ_K3_FW
-#define SJ_K3_FW 4   // warps (= units of two chunks) per CTA of the flatten kernel (2 and 4 measure alike, 8: -4 %)
-#endif
-
 using namespace sjb200;
 
 namespace {
@@ -29,6 +25,8 @@ constexpr uint64_t MIN_TILE = 2 * 2048;
 // round 2 and removed again: profiles/r2_overlap_experiments.txt.)
 constexpr uint64_t SPLIT_MIN_BYTES = 24ull << 20;
 constexpr uint64_t STREAM_MIN_BYTES = 80ull << 20;
+constexpr int FLATTEN_FW = 4;   // warps (= units of two chunks) per CTA of the flatten kernel (2 and 4 measure alike, 8: -4 %)
+constexpr int STREAM_NW = 8;    // compute warps per CTA of the stream classify kernel
 
 inline int32_t cuda_err(cudaError_t e) {
     if (e == cudaSuccess) return SJB200_SUCCESS;
@@ -42,30 +40,7 @@ inline int32_t cuda_err(cudaError_t e) {
         if (e__ != cudaSuccess) return cuda_err(e__); \
     } while (0)
 
-// Tuning knobs from the environment, read ONCE (first context creation), never on the call path.
-struct Knobs {
-    int pdl = 1;            // SJB200_PDL=0: no programmatic dependent launch between the launches of a document
-    int warps = 0;          // SJB200_WARPS: tile shape of the persistent kernel (2/4/8/16/24)
-    int kernel = SJB200_KERNEL_AUTO;   // SJB200_KERNEL=persist|split|stream
-    uint64_t chunk_bytes = 32ull << 20;   // SJB200_CHUNK_MIB: chunk size of the streaming host path
-};
 bool valid_warps(int w) { return w == 2 || w == 4 || w == 8 || w == 16 || w == 24; }
-const Knobs &knobs() {
-    static const Knobs k = [] {
-        Knobs v;
-        if (const char *e = getenv("SJB200_PDL")) v.pdl = atoi(e);
-        if (const char *e = getenv("SJB200_WARPS")) v.warps = valid_warps(atoi(e)) ? atoi(e) : 0;
-        if (const char *e = getenv("SJB200_KERNEL")) {
-            if (strcmp(e, "persist") == 0) v.kernel = SJB200_KERNEL_PERSISTENT;
-            if (strcmp(e, "split") == 0) v.kernel = SJB200_KERNEL_SPLIT;
-            if (strcmp(e, "stream") == 0) v.kernel = SJB200_KERNEL_STREAM;
-        }
-        if (const char *e = getenv("SJB200_CHUNK_MIB"))
-            if (atoi(e) > 0) v.chunk_bytes = (uint64_t)atoi(e) << 20;
-        return v;
-    }();
-    return k;
-}
 
 }  // namespace
 
@@ -142,19 +117,15 @@ cudaError_t prepare_persist(int *occ) {
 template <int NW>
 cudaError_t prepare_split(int *occ) {
     using Cfg = SplitCfg<NW>;
-    cudaFuncSetAttribute(stage1_flatten2_kernel<SJ_K3_FW>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(stage1_flatten2_kernel<FLATTEN_FW>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     return prepare_kernel(stage1_classify_kernel<NW, true>, stage1_classify_kernel<NW, false>, Cfg::THREADS, Cfg::SMEM_BYTES, occ);
 }
-#ifndef SJ_STREAM_NW
-#define SJ_STREAM_NW 8
-#endif
-constexpr int STREAM_NW = SJ_STREAM_NW;
 cudaError_t prepare_stream(int *occ) {
     using Cfg = StreamCfg<STREAM_NW>;
     // every kernel of the pipeline asks for the same shared-memory carve-out: kernels with different L1 / shared splits
     // cannot share an SM, and scan + flatten of one window must run beside the classify CTAs of the next
     cudaFuncSetAttribute(stage1_span_scan_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    cudaFuncSetAttribute(stage1_flatten2_kernel<SJ_K3_FW>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(stage1_flatten2_kernel<FLATTEN_FW>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     return prepare_kernel(stage1_stream_classify_kernel<STREAM_NW, true>, stage1_stream_classify_kernel<STREAM_NW, false>, Cfg::THREADS, Cfg::SMEM_BYTES, occ);
 }
 // Launch `kernel` so that it may be scheduled while the previous kernel of the stream drains (programmatic dependent
@@ -179,12 +150,12 @@ cudaError_t launch_persist(const Stage1Params &p, cudaStream_t s, int max_ctas) 
     const unsigned span = p.tile_end - p.tile_begin;
     const unsigned grid = span < (unsigned)max_ctas ? span : (unsigned)max_ctas;
     // as the fallback of the stream pipeline (spec_flag set) it follows the flatten kernel as a dependent launch
-    return launch_dependent(stage1_persistent_kernel<NW, UTF8>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, s, p.spec_flag != nullptr && knobs().pdl != 0, p);
+    return launch_dependent(stage1_persistent_kernel<NW, UTF8>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, s, p.spec_flag != nullptr, p);
 }
 // flatten chunks [c0, c1) (c0 even): units of two chunks per warp
-cudaError_t launch_flatten(const Stage1Params &p, uint32_t c0, uint32_t c1, cudaStream_t s, bool pdl) {
-    constexpr int FW = SJ_K3_FW;
-    return launch_dependent(stage1_flatten2_kernel<FW>, (c1 - c0 + FW * 2 - 1) / (FW * 2), Flatten2Cfg<FW>::THREADS, Flatten2Cfg<FW>::SMEM_BYTES, s, pdl, p, c0, c1);
+cudaError_t launch_flatten(const Stage1Params &p, uint32_t c0, uint32_t c1, cudaStream_t s) {
+    constexpr int FW = FLATTEN_FW;
+    return launch_dependent(stage1_flatten2_kernel<FW>, (c1 - c0 + FW * 2 - 1) / (FW * 2), Flatten2Cfg<FW>::THREADS, Flatten2Cfg<FW>::SMEM_BYTES, s, true, p, c0, c1);
 }
 
 template <int NW, bool UTF8>
@@ -196,29 +167,27 @@ cudaError_t launch_split(const Stage1Params &p, cudaStream_t s, int max_ctas) {
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const uint32_t c0 = p.tile_begin * NW, c1 = p.tile_end * NW;
-    return launch_flatten(p, c0, c1, s, knobs().pdl != 0);
+    return launch_flatten(p, c0, c1, s);
 }
 // The stream pipeline (stage1_stream.cuh): classify -> span_scan -> flatten, stream ordered; the dependent
 // launches overlap their launch latency with their predecessor (programmatic dependent launch).
 template <bool UTF8>
 cudaError_t launch_stream(sjb200_ctx *c, const Stage1Params &p, cudaStream_t s, int max_ctas) {
     using Cfg = StreamCfg<STREAM_NW>;
-    const bool pdl = knobs().pdl != 0;
     const uint32_t nchunks = (uint32_t)((p.alen + 2047) / 2048);
     const unsigned want = (nchunks + STREAM_NW - 1) / STREAM_NW;
     const unsigned grid = want < (unsigned)max_ctas ? want : (unsigned)max_ctas;
     // (the first launch of a document is a dependent launch too: back-to-back documents overlap their launch latencies)
-    cudaError_t e = launch_dependent(stage1_stream_classify_kernel<STREAM_NW, UTF8>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, s, pdl, p, nchunks, 0u, nchunks, p.abase - Cfg::HALO);
+    cudaError_t e = launch_dependent(stage1_stream_classify_kernel<STREAM_NW, UTF8>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, s, true, p, nchunks, 0u, nchunks, p.abase - Cfg::HALO);
     const unsigned nblocks = (nchunks + SPAN_BLOCK - 1) / SPAN_BLOCK;
-    if (e == cudaSuccess) e = launch_dependent(stage1_span_scan_kernel, nblocks, SPAN_SCAN_THREADS, 0, s, pdl, p, nchunks);
-    if (e == cudaSuccess) e = launch_flatten(p, 0u, nchunks, s, pdl);
+    if (e == cudaSuccess) e = launch_dependent(stage1_span_scan_kernel, nblocks, SPAN_SCAN_THREADS, 0, s, true, p, nchunks);
+    if (e == cudaSuccess) e = launch_flatten(p, 0u, nchunks, s);
     c->launches += 3;
     return e;
 }
 
 int pick_warps(const sjb200_ctx *c, uint64_t alen) {
     if (c->forced_warps) return c->forced_warps;
-    if (knobs().warps) return knobs().warps;
     // small documents: smaller tiles so that the work spreads over all 148 SMs (measured, tools/quickbench.py: 16-warp tiles
     // win from 8 MiB on -- 8 MiB: 480 vs 411 GB/s, 16 MiB: 761 vs 718, 48 MiB: 1060 vs 996)
     if (alen >= (uint64_t)8 << 20) return 16;
@@ -298,7 +267,7 @@ int32_t plan_document(sjb200_ctx *c, DocPlan &d, const uint8_t *d_buf, uint64_t 
     p.gen = c->gen;
     p.flags = flags;
     d.utf8 = !(flags & SJB200_FLAG_NO_UTF8);
-    int kind = c->kernel_kind != SJB200_KERNEL_AUTO ? c->kernel_kind : knobs().kernel;
+    int kind = c->kernel_kind;
     const bool auto_kind = kind == SJB200_KERNEL_AUTO;
     if (auto_kind) {
         kind = SJB200_KERNEL_PERSISTENT;
@@ -309,7 +278,7 @@ int32_t plan_document(sjb200_ctx *c, DocPlan &d, const uint8_t *d_buf, uint64_t 
     if (kind == SJB200_KERNEL_SPLIT && d.warps != 8 && d.warps != 16) {
         // the split pair exists for 8- and 16-warp tiles only: an explicit shape it does not have is an error, never a silent
         // substitution of another kernel shape
-        if (c->forced_warps || knobs().warps) {
+        if (c->forced_warps) {
             if (!auto_kind) return SJB200_UNEXPECTED_ERROR;
             kind = SJB200_KERNEL_PERSISTENT;   // chosen automatically: the persistent kernel has every shape
         } else {
@@ -625,7 +594,6 @@ int32_t sjb200_ctx_create(int32_t device, uint64_t max_len, uint64_t max_len_hos
     for (int k = 0; k < sjb200_ctx::MAX_CHUNKS && e == cudaSuccess; k++) e = cudaEventCreateWithFlags(&c->chunk_ev[k], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaHostAlloc(&c->h_progress, 4 * sjb200_ctx::MAX_CHUNKS, cudaHostAllocMapped);
     if (e == cudaSuccess) e = cudaHostGetDevicePointer(&c->d_progress, c->h_progress, 0);
-    c->chunk_bytes = knobs().chunk_bytes;
     if (e == cudaSuccess) e = cudaEventCreate(&c->ev0);
     if (e == cudaSuccess) e = cudaEventCreate(&c->ev1);
     if (e == cudaSuccess) e = prepare_persist<2>(&c->persist_occ[0]);

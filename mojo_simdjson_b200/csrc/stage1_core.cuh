@@ -22,9 +22,6 @@
 #pragma once
 #include <stdint.h>
 
-#ifndef SJ_SHR_FMA
-#define SJ_SHR_FMA 1
-#endif
 #if defined(__CUDACC__)
 #define SJ_HD __host__ __device__ __forceinline__
 #else
@@ -113,7 +110,7 @@ SJ_HD uint32_t bitselect(uint32_t a, uint32_t b, uint32_t m) {
 }
 // x >> s on the FMA pipe (IMAD.HI): the ALU pipe is the one this kernel saturates (profiles/b200_pipe_throughput_ubench.txt)
 SJ_HD uint32_t shr_fma(uint32_t x, int s) {
-#if defined(__CUDA_ARCH__) && SJ_SHR_FMA
+#if defined(__CUDA_ARCH__)
     return __umulhi(x, 1u << (32 - s));
 #else
     return x >> s;

@@ -17,22 +17,8 @@
 
 #include "stage1_core.cuh"
 
-// experiment knobs (defaults = the shipped configuration)
-#ifndef SJ_MBAR_HINT
-#define SJ_MBAR_HINT 0
-#endif
-#ifndef SJ_NSLEEP
-#define SJ_NSLEEP 20
-#endif
-#ifndef SJ_REG8
-#define SJ_REG8 56
-#endif
-#ifndef SJ_REG16
-#define SJ_REG16 56
-#endif
-#ifndef SJ_REG24
-#define SJ_REG24 72
-#endif
+// -DSJ_TRACE=1: per-tile timeline of the persistent kernel (sjb200_debug_trace).  The split pair's classify kernel shares
+// its tile fetch and aggregate steps (stage1_persistent.cuh), so in such builds it fills slots 0 and 2 of its tiles too.
 #ifndef SJ_TRACE
 #define SJ_TRACE 0
 #endif
@@ -130,21 +116,17 @@ __device__ __forceinline__ void bulk_load(uint32_t dst, const void *src, uint32_
                  : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    // try_wait suspends the thread in hardware until the phase completes or the time hint expires (no busy spin)
+    // try_wait suspends the thread in hardware until the phase completes or a system-dependent time limit expires (no busy spin)
     asm volatile(
         "{\n"
         ".reg .pred p;\n"
         "SJ_WAIT:\n"
-#if SJ_MBAR_HINT
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-#else
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-#endif
         "@p bra SJ_DONE;\n"
         "bra SJ_WAIT;\n"
         "SJ_DONE:\n"
         "}\n" ::"r"(bar),
-        "r"(parity), "r"((uint32_t)SJ_MBAR_HINT)
+        "r"(parity)
         : "memory");
 }
 __device__ __forceinline__ uint64_t ld_desc(const uint64_t *p) {
@@ -155,11 +137,13 @@ __device__ __forceinline__ uint64_t ld_desc(const uint64_t *p) {
 __device__ __forceinline__ void st_desc(uint64_t *p, uint64_t v) {
     asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
+// back-off between two polls of a look-back descriptor (ns)
+constexpr unsigned DESC_POLL_NS = 20;
 // spin until tile j has published something for this generation
 __device__ __forceinline__ uint64_t wait_desc(const uint64_t *desc, int j, uint32_t gen) {
     uint64_t d = ld_desc(desc + j);
     while (desc_gen(d) != (gen & GEN_MASK)) {
-        __nanosleep(SJ_NSLEEP);
+        __nanosleep(DESC_POLL_NS);
         d = ld_desc(desc + j);
     }
     return d;
@@ -244,7 +228,7 @@ __device__ __forceinline__ LookbackResult lookback(const uint64_t *desc, uint32_
         uint32_t st = DESC_PREFIX;  // before the first tile: outside a string, nothing produced
         if (j >= 0) {
             while (desc_gen(d) != want) {
-                __nanosleep(SJ_NSLEEP);
+                __nanosleep(DESC_POLL_NS);
                 d = ld_desc(desc + j);
             }
             st = desc_status(d);
@@ -337,9 +321,7 @@ __device__ __forceinline__ void warp_load(LaneInput &in, const uint8_t *smem_til
 // lane, its end-of-document bit: 80 B) in the warp's own shared-memory slots and report them; the same warp validates them
 // 32 at a time at the end of its run of chunks (stage1_stream.cuh: validate_parked_lanes).  `u8_slots` points at the
 // first free slot.  DEFER_U8 == 0: always validate inline.
-#ifndef SJ_U8_DEFER_MAX
-#define SJ_U8_DEFER_MAX 8
-#endif
+constexpr int U8_DEFER_MAX = 8;   // most lanes of a chunk that DEFER_U8 parks
 template <bool UTF8, int DEFER_U8 = 0>
 __device__ __forceinline__ void warp_compute(LanePhase1 &r, const LaneInput &in, int lane, const Stage1Params &P,
                                              uint4 *u8_slots = nullptr /* DEFER_U8: the warp's free shared-memory slots, 5 uint4 each */,
@@ -365,7 +347,7 @@ __device__ __forceinline__ void warp_compute(LanePhase1 &r, const LaneInput &in,
             const bool any_hi = ((pl[7] | ph[7]) != 0) || ((in.prev & 0x80808080u) != 0);
             const uint32_t hi_lanes = __ballot_sync(0xFFFFFFFFu, any_hi);
             r.u8_lanes = 0;
-            if (DEFER_U8 && __popc(hi_lanes) <= SJ_U8_DEFER_MAX) {
+            if (DEFER_U8 && __popc(hi_lanes) <= U8_DEFER_MAX) {
                 // the k-th flagged lane parks its bit planes, the 4 bytes before it and its end-of-document bit in slot k
                 r.u8_lanes = hi_lanes;
                 if (any_hi) {
@@ -523,10 +505,12 @@ __device__ __forceinline__ void flatten_word_pair(uint32_t sptr, uint32_t bits, 
         : "memory");
 }
 
-// stage[a .. a+total) -> out[first .. first+total) by one warp, total <= 512: at most four predicated 16-byte copies per
-// lane plus the ragged head / tail entries (a = phase of `first` in its 16-byte line, so stage and out are congruent)
-__device__ __forceinline__ void copy_out_warp(const uint32_t *stage, uint32_t a, uint32_t total, uint32_t *out, uint64_t first,
-                                              uint64_t cap, uint32_t lane) {
+// stage[a .. a+total) -> out[first .. first+total) by one warp, a + total < 4 * NV + 4: up to NV 16-byte copies, the lanes'
+// predicated ones unrolled, plus the ragged head / tail entries (a = phase of `first` in its 16-byte line, so stage and out
+// are congruent)
+template <int NV>
+__device__ __forceinline__ void copy_out_warp_n(const uint32_t *stage, uint32_t a, uint32_t total, uint32_t *out, uint64_t first,
+                                                uint64_t cap, uint32_t lane) {
     const uint32_t end = a + total;
     uint32_t *g0 = out + ((int64_t)first - (int64_t)a);   // 16-byte aligned, may point below `out` by up to 3 entries
     if (first + total <= cap) {
@@ -535,7 +519,7 @@ __device__ __forceinline__ void copy_out_warp(const uint32_t *stage, uint32_t a,
         const uint4 *sv = reinterpret_cast<const uint4 *>(stage) + lane;
         uint4 *gv = reinterpret_cast<uint4 *>(g0) + lane;
 #pragma unroll
-        for (int k = 0; k < 4; k++) {
+        for (int k = 0; k < (NV + 31) / 32; k++) {
             const uint32_t v = lane + 32u * k;
             if (v - v_lo < nvec) gv[32 * k] = sv[32 * k];          // v_lo <= v < v_hi in one unsigned compare
         }

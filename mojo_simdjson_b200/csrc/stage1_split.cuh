@@ -1,6 +1,6 @@
 // stage1_split.cuh -- stage 1 as two launches for large documents: classify, then flatten.
 //
-// The fused kernels (stage1_persistent.cuh, stage1_dataflow.cuh) are bound by latency, not by a pipe: a warp that
+// The persistent kernel (stage1_persistent.cuh) is bound by latency, not by a pipe: a warp that
 // classifies 2 KiB and then extracts its indexes spends long stretches waiting (bulk copy, look-back, the serial
 // clear-lowest-bit chain of the extraction loop), and registers cap the SM at ~34 such warps.  Measured standalone
 // (tools/ubench_stages.cu) both halves only reach their issue-bound rate with >= 32 warps per SM *each*.  So for
@@ -8,24 +8,22 @@
 // register budget allows, and neither ever waits for a carry:
 //
 //   stage1_classify_kernel : persistent CTAs of NW compute warps + 1 scan warp, tiles drawn from the ticket counter
-//                            exactly as in the fused kernel.  A compute warp turns 2 KiB into the two structural masks
+//                            exactly as in the persistent kernel.  A compute warp turns 2 KiB into the two structural masks
 //                            (string state entering the chunk unknown -> one mask per parity), stores both (16 bytes per
 //                            64 input bytes) and moves on.  The scan warp runs the decoupled look-back for every tile
 //                            and leaves, per 2 KiB chunk, one 8-byte carry word: bit 63 = chunk starts inside a string,
 //                            bits 0..39 = rank of its first structural in the output.  It also writes the verdict.
+//                            (Fetch, aggregate and prefix steps are shared with the persistent kernel; in -DSJ_TRACE=1
+//                            builds they fill trace slots 0 and 2 of this kernel's tiles.)
 //   stage1_flatten2_kernel : one warp per unit of two chunks, no shared state between warps: carry word -> pick the mask
 //                            plane -> every lane extracts the same number of consecutive indexes (balanced, see below)
 //                            into the warp's staging area, 16-byte stores.
 //
 // Extra HBM traffic: the mask planes, 16 B written + 8 B read per 64 input bytes (+23 % over the algorithmic bytes at the
 // bench document's density of 0.161 structurals per byte).
-// Same arithmetic, same descriptors, same results as the fused kernels (reference json_structural_indexer.mojo:83-186).
+// Same arithmetic, same descriptors, same results as the persistent kernel (reference json_structural_indexer.mojo:83-186).
 #pragma once
 #include "stage1_persistent.cuh"
-
-#ifndef SJ_SPLITREG
-#define SJ_SPLITREG 56  // registers per thread of the classify kernel
-#endif
 
 namespace sjb200 {
 
@@ -41,16 +39,7 @@ struct SplitCfg {
     static constexpr int NIN = 2;                                         // input buffers (bulk copy of tile i+2 overlaps tile i+1)
     static constexpr int IN_STRIDE = ((16 + TILE) + 127) & ~127;          // halo + tile
     static constexpr int SMEM_BYTES = NIN * IN_STRIDE;
-    static constexpr int MAXREG = SJ_SPLITREG;
-};
-
-struct SplitSlot {                // hand-off from the compute warps to the scan warp
-    uint32_t wc0[32], wc1[32], wflags[32];
-    uint32_t R[32], off0[32], off1[32];
-    uint64_t agg;
-    uint32_t tail;
-    uint32_t arrived;
-    int32_t tile;
+    static constexpr int MAXREG = 56;                                    // registers per thread of the classify kernel
 };
 
 template <int NW, bool UTF8>
@@ -61,7 +50,7 @@ __global__ void __launch_bounds__((NW + 1) * 32) __maxnreg__(SplitCfg<NW>::MAXRE
     constexpr int NS = 4;
     extern __shared__ __align__(128) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t s_bar[NIN + 2 * NS];   // in_full[NIN], sum_full[NS], slot_free[NS]
-    __shared__ SplitSlot s_slot[NS];
+    __shared__ TileSlot s_slot[NS];
     __shared__ int32_t s_tile_of[NIN];
     __shared__ uint32_t s_loaded[NIN];
 
@@ -87,21 +76,8 @@ __global__ void __launch_bounds__((NW + 1) * 32) __maxnreg__(SplitCfg<NW>::MAXRE
     // draw the ticket of iteration `it` and start its bulk copy into input buffer it % NIN (free by construction)
     auto produce = [&](int it) {
         const int b = it % NIN;
-        const uint32_t k = P.tile_begin + atomicAdd(ticket, 1u);
-        if (k < P.tile_end) {
-            const int t = (int)k;
-            s_tile_of[b] = t;
-            const int64_t tb = (int64_t)t * TILE;
-            int64_t nbytes = (int64_t)P.alen - tb;
-            nbytes = nbytes > TILE ? TILE : nbytes;
-            nbytes = (nbytes + 15) & ~15ll;
-            const uint32_t halo = t > 0 ? 16u : 0u;
-            mbar_expect_tx(bar_in + 8 * b, (uint32_t)nbytes + halo);
-            bulk_load(smem_u32(smem_raw) + b * Cfg::IN_STRIDE + 16u - halo, P.abase + tb - halo, (uint32_t)nbytes + halo, bar_in + 8 * b);
-        } else {
-            s_tile_of[b] = -1;
-            mbar_arrive(bar_in + 8 * b);
-        }
+        if (!fetch_tile<TILE>(P, ticket, s_tile_of[b], smem_u32(smem_raw) + b * Cfg::IN_STRIDE, bar_in + 8 * b))
+            mbar_arrive(bar_in + 8 * b);   // no more work
     };
     if (tid == 0) {
         for (int k = 0; k < NIN; k++) produce(k);
@@ -112,7 +88,7 @@ __global__ void __launch_bounds__((NW + 1) * 32) __maxnreg__(SplitCfg<NW>::MAXRE
         for (int i = 0;; i++) {
             const int slot = i & (NS - 1);
             mbar_wait(bar_sum + 8 * slot, (uint32_t)(i / NS) & 1u);
-            SplitSlot &S = s_slot[slot];
+            TileSlot &S = s_slot[slot];
             const int cur = *reinterpret_cast<volatile int32_t *>(&S.tile);
             if (cur < 0) break;
             const TileAgg agg = desc_unpack_agg(S.agg);
@@ -120,24 +96,10 @@ __global__ void __launch_bounds__((NW + 1) * 32) __maxnreg__(SplitCfg<NW>::MAXRE
             const uint32_t R = have ? S.R[lane] : 0u, off0 = have ? S.off0[lane] : 0u, off1 = have ? S.off1[lane] : 0u;
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_free + 8 * slot);   // everything we need is in registers: the slot may be reused
-            LookbackResult lb = {0, 0, 0};
-            if (cur > 0) lb = lookback(P.desc, P.gen, cur, lane);
-            const uint32_t s_in = lb.s_in & 1u;
-            const uint32_t total = s_in ? agg.c[1] : agg.c[0];
-            TilePrefix pre;
-            pre.s_out = s_in ^ agg.par;
-            pre.e_out = agg.e_out;
-            pre.p_out = agg.p_out;
-            pre.err = lb.err | ((s_in ? agg.un[1] : agg.un[0]) ? EF_UNESCAPED : 0u) | (agg.u8 ? EF_UTF8 : 0u);
-            pre.count = lb.base + total;
-            if (lane == 0) {
-                st_desc(P.desc + cur, desc_pack_prefix(P.gen, pre));
-                if (cur == (int)P.tile_end - 1 && P.progress) *P.progress = pre.count;
-                if (cur == (int)P.ntiles - 1) write_verdict(P, pre);
-            }
+            const TileStart st = publish_tile_prefix(P, agg, cur, lane);
             if (have) {
-                const uint64_t first = (uint64_t)lb.base + (s_in ? off1 : off0);
-                P.carry[(size_t)cur * NW + lane] = first | (((s_in ^ R) & 1u) ? CARRY_INSIDE : 0ull);
+                const uint64_t first = (uint64_t)st.base + (st.s_in ? off1 : off0);
+                P.carry[(size_t)cur * NW + lane] = first | (((st.s_in ^ R) & 1u) ? CARRY_INSIDE : 0ull);
             }
         }
     } else {
@@ -171,38 +133,7 @@ __global__ void __launch_bounds__((NW + 1) * 32) __maxnreg__(SplitCfg<NW>::MAXRE
                 __stcs(reinterpret_cast<unsigned long long *>(mp + 32), (unsigned long long)ph.m1);
             }
             if (i >= NS) mbar_wait(bar_free + 8 * slot, (uint32_t)(i / NS - 1) & 1u);   // the scan warp is done with iteration i - NS
-            SplitSlot &S = s_slot[slot];
-            uint32_t order = 0;
-            if (lane == 0) {
-                S.wc0[warp] = ph.wc0;
-                S.wc1[warp] = ph.wc1;
-                S.wflags[warp] = ph.wflags;
-                if (warp == NW - 1) S.tail = ph.tail;
-                __threadfence_block();
-                order = atomicAdd(&S.arrived, 1u);
-            }
-            order = __shfl_sync(0xFFFFFFFFu, order, 0);
-            if (order == NW - 1) {
-                __threadfence_block();
-                const bool have = lane < NW;
-                uint32_t R, off0, off1;
-                const TileAgg agg = tile_aggregate(have ? S.wflags[lane] : 0u, have ? S.wc0[lane] : 0u, have ? S.wc1[lane] : 0u,
-                                                   S.tail, NW, lane, R, off0, off1);
-                if (have) {
-                    S.R[lane] = R;
-                    S.off0[lane] = off0;
-                    S.off1[lane] = off1;
-                }
-                const uint64_t packed = desc_pack_agg(P.gen, agg);
-                if (lane == 0) {
-                    if (tile > 0) st_desc(P.desc + tile, packed);
-                    S.agg = packed;
-                    S.tile = tile;
-                    S.arrived = 0;
-                }
-                __syncwarp();
-                if (lane == 0) mbar_arrive(bar_sum + 8 * slot);
-            }
+            publish_tile_aggregate<NW>(s_slot[slot], ph, warp, lane, tile, P, bar_sum + 8 * slot);
             i++;
         }
         if (warp == 0 && lane == 0) {   // tell the scan warp that iteration i does not exist
@@ -231,7 +162,7 @@ __device__ __forceinline__ void flatten_chunk(const Stage1Params &P, uint32_t c,
         flatten_word_pair(sp, lo, v0 + 31u);
         flatten_word_pair(sp + 4u * cnt_lo, hi, v0 + 63u);   // (the popcount of the low word is needed for the scan anyway)
         __syncwarp();
-        copy_out_warp(stage, a, wtotal, P.out, first, P.cap, (uint32_t)lane);
+        copy_out_warp_n<128>(stage, a, wtotal, P.out, first, P.cap, (uint32_t)lane);
     } else {
         flatten_direct(P.out, P.cap, first + (incl - cnt), structural, v0);
     }
@@ -254,16 +185,11 @@ __device__ __forceinline__ void flatten_chunk(const Stage1Params &P, uint32_t c,
 // Units with more than CAP indexes (denser than 0.19 structurals per byte) take the per-chunk path (flatten_chunk).
 // BitIndexer.write, reference json_structural_indexer.mojo:46-58.
 // ---------------------------------------------------------------------------------------------
-#ifndef SJ_FL2_CAP
-#define SJ_FL2_CAP 768
-#endif
-#ifndef SJ_FL2_MINCTAS
-#define SJ_FL2_MINCTAS 11
-#endif
 template <int FW>
 struct Flatten2Cfg {
     static constexpr int THREADS = FW * 32;
-    static constexpr int CAP = SJ_FL2_CAP;                         // indexes of a unit flattened through the balanced path
+    static constexpr int MIN_CTAS = 11;                           // resident CTAs per SM the register budget must allow
+    static constexpr int CAP = 768;                               // indexes of a unit flattened through the balanced path
     static constexpr int QMAX = ((CAP + 31) / 32) | 1;            // trips per lane (odd)
     static constexpr int STAGE = 32 * QMAX + 4;                   // every lane writes q slots (the last ones past K) + output phase
     static constexpr int NVEC = (CAP + 3 + 3) / 4;                // 16-byte vectors the copy-out may have to move
@@ -311,42 +237,13 @@ __device__ __forceinline__ void flatten_balanced_loop(uint32_t w, uint32_t vb, u
         : "memory");
 }
 
-// stage[a .. a+total) -> out[first .. first+total) by one warp, total <= 4 * NV - 6: NV predicated 16-byte copies per lane
-// plus the ragged head / tail entries (a = phase of `first` in its 16-byte line, so stage and out are congruent)
-template <int NV>
-__device__ __forceinline__ void copy_out_warp_n(const uint32_t *stage, uint32_t a, uint32_t total, uint32_t *out, uint64_t first,
-                                                uint64_t cap, uint32_t lane) {
-    const uint32_t end = a + total;
-    uint32_t *g0 = out + ((int64_t)first - (int64_t)a);   // 16-byte aligned, may point below `out` by up to 3 entries
-    if (first + total <= cap) {
-        const uint32_t v_lo = (a + 3u) >> 2, v_hi = end >> 2;
-        const uint32_t nvec = v_hi > v_lo ? v_hi - v_lo : 0u;      // whole vectors; none when the run is shorter than a line
-        const uint4 *sv = reinterpret_cast<const uint4 *>(stage) + lane;
-        uint4 *gv = reinterpret_cast<uint4 *>(g0) + lane;
-#pragma unroll
-        for (int k = 0; k < (NV + 31) / 32; k++) {
-            const uint32_t v = lane + 32u * k;
-            if (v - v_lo < nvec) gv[32 * k] = sv[32 * k];          // v_lo <= v < v_hi in one unsigned compare
-        }
-        if (lane < 8u) {
-            const uint32_t j = lane < 4u ? lane : 4u * v_hi + (lane - 4u);
-            const bool head = lane < 4u && j >= a && j < end && j < 4u * v_lo;
-            const bool tail = lane >= 4u && j < end && j >= a && v_hi >= v_lo;
-            if (head || tail) g0[j] = stage[j];
-        }
-    } else {
-        for (uint32_t j = a + lane; j < end; j += 32u)
-            if (first + (j - a) < cap) g0[j] = stage[j];
-    }
-}
-
 __device__ __forceinline__ void sts_u2(uint32_t a, uint32_t x, uint32_t y) {
     asm volatile("st.shared.v2.u32 [%0], {%1,%2};" ::"r"(a), "r"(x), "r"(y) : "memory");
 }
 
 // units of two chunks in [chunk_begin, chunk_end): unit u = chunks chunk_begin + 2u and + 1 (the last one may be missing)
 template <int FW>
-__global__ void __launch_bounds__(FW * 32, SJ_FL2_MINCTAS) stage1_flatten2_kernel(const Stage1Params P, uint32_t chunk_begin, uint32_t chunk_end) {
+__global__ void __launch_bounds__(FW * 32, Flatten2Cfg<FW>::MIN_CTAS) stage1_flatten2_kernel(const Stage1Params P, uint32_t chunk_begin, uint32_t chunk_end) {
     using Cfg = Flatten2Cfg<FW>;
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;

@@ -27,30 +27,12 @@
 #pragma once
 #include "stage1_split.cuh"
 
-#ifndef SJ_STREAMREG
-#define SJ_STREAMREG 64
-#endif
-#ifndef SJ_STREAM_DEPTH
-#define SJ_STREAM_DEPTH 2
-#endif
-#ifndef SJ_TICKET_CHUNKS
-#define SJ_TICKET_CHUNKS 4
-#endif
-#ifndef SJ_MASK_STORE
-#define SJ_MASK_STORE 1   // 1: streaming stores (the planes of a large document do not fit the L2 anyway), 0: write-back stores
-#endif
-
 namespace sjb200 {
 
 #if defined(__CUDACC__)
 
-__device__ __forceinline__ void st_mask(uint64_t *p, uint64_t v) {
-#if SJ_MASK_STORE
-    __stcs(reinterpret_cast<unsigned long long *>(p), (unsigned long long)v);
-#else
-    *p = v;
-#endif
-}
+// streaming stores: the planes of a large document do not fit the L2 anyway
+__device__ __forceinline__ void st_mask(uint64_t *p, uint64_t v) { __stcs(reinterpret_cast<unsigned long long *>(p), (unsigned long long)v); }
 
 // One thread draws from the chunk counter.  Plain PTX: atomicAdd() makes the compiler aggregate over the active lanes (vote,
 // elect, shuffle), and that shuffle waits for the atomic at once -- here its result is not needed before the next run.
@@ -63,13 +45,13 @@ __device__ __forceinline__ uint32_t ticket_draw(uint32_t *counter, uint32_t n) {
 template <int NW>
 struct StreamCfg {
     static constexpr int THREADS = NW * 32;
-    static constexpr int DEPTH = SJ_STREAM_DEPTH;
+    static constexpr int DEPTH = 2;                         // chunks in flight per warp
     static constexpr int HALO = 32;
     static constexpr int BUF = 2048 + HALO;                 // 16-byte multiple
-    static constexpr int PARK = 32 * 80;                    // 32 parked UTF-8 lanes of 80 B per warp; validated when fewer than SJ_U8_DEFER_MAX slots are left
+    static constexpr int PARK = 32 * 80;                    // 32 parked UTF-8 lanes of 80 B per warp; validated when fewer than U8_DEFER_MAX slots are left
     static constexpr int WARP_BYTES = DEPTH * BUF + PARK;
     static constexpr int SMEM_BYTES = NW * WARP_BYTES;
-    static constexpr int MAXREG = SJ_STREAMREG;
+    static constexpr int MAXREG = 64;
 };
 
 // phase 1 input of one lane from the warp's private buffer; `chunk` is the shared-space address of the chunk's first byte, HALO
@@ -208,7 +190,7 @@ __device__ __forceinline__ bool resolve_long_runs(const Stage1Params &P, uint32_
 // kernel that follows resets it).  A static partition would be slightly cheaper but assumes that every CTA of the grid is
 // resident from the start: with another kernel on the device (the NCCL verdict exchange of the previous pass, a second
 // context) a displaced CTA would start only when some other CTA has finished its whole share, doubling the kernel time.
-constexpr uint32_t TICKET_CHUNKS = SJ_TICKET_CHUNKS;
+constexpr uint32_t TICKET_CHUNKS = 4;
 constexpr uint32_t NO_CHUNK = 0xFFFFFFFFu;
 
 // validates the `parked` lanes a warp left in its shared-memory slots (80 B each: 16 bit-plane words, the 4 bytes before the
@@ -244,7 +226,7 @@ __global__ void __launch_bounds__(NW * 32) __maxnreg__(StreamCfg<NW>::MAXREG) st
                                                                                                             const uint8_t *src0 /* P.abase - HALO */) {
     using Cfg = StreamCfg<NW>;
     constexpr int DEPTH = Cfg::DEPTH;
-    static_assert(SJ_U8_DEFER_MAX <= 32, "a chunk must not park more lanes than the warp's slots hold");
+    static_assert(U8_DEFER_MAX <= 32, "a chunk must not park more lanes than the warp's slots hold");
     extern __shared__ __align__(128) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t s_bar[NW * DEPTH];
     // the lane number is read once (volatile: the compiler would otherwise re-derive it from %tid inside the loop, a
@@ -341,7 +323,7 @@ __global__ void __launch_bounds__(NW * 32) __maxnreg__(StreamCfg<NW>::MAXREG) st
             st_mask(mp, ph.m0);
             st_mask(mp + 32, ph.m1);
             if (lane == 0) reinterpret_cast<uint4 *>(P.chunk_sum)[c] = make_uint4(ph.wc0, ph.wc1, ph.wflags, 0u);
-            if (UTF8 && parked > 32u - SJ_U8_DEFER_MAX) {
+            if (UTF8 && parked > 32u - U8_DEFER_MAX) {
                 // the next chunk might not find room: the lanes whose validation was deferred, up to 32 at a time
                 __syncwarp();
                 u8_bad |= validate_parked_lanes(park, parked, lane);
@@ -398,10 +380,7 @@ __device__ __forceinline__ SpanAcc warp_span_inclusive(SpanAcc a, int lane) {
     }
     return a;
 }
-#ifndef SJ_SCAN_THREADS
-#define SJ_SCAN_THREADS 1024
-#endif
-constexpr uint32_t SPAN_SCAN_THREADS = SJ_SCAN_THREADS;
+constexpr uint32_t SPAN_SCAN_THREADS = 1024;
 // inclusive scan over the CTA's threads in thread order; returns this thread's inclusive span, `total` = the CTA's
 __device__ __forceinline__ SpanAcc block_span_inclusive(const SpanAcc mine, uint4 *s_w /* [32] */, SpanAcc &total) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -421,10 +400,7 @@ __device__ __forceinline__ SpanAcc block_span_inclusive(const SpanAcc mine, uint
     return a;
 }
 
-#ifndef SJ_SPAN_PER_THREAD
-#define SJ_SPAN_PER_THREAD 4
-#endif
-constexpr int SPAN_PER_THREAD = SJ_SPAN_PER_THREAD;        // consecutive chunk summaries per thread
+constexpr int SPAN_PER_THREAD = 4;        // consecutive chunk summaries per thread
 constexpr uint32_t SPAN_BLOCK = SPAN_SCAN_THREADS * SPAN_PER_THREAD;   // chunk summaries per CTA (8 MiB of input)
 
 // One launch, one CTA per SPAN_BLOCK chunk summaries (8 MiB of input): local ordered reduction -> the block aggregate,
@@ -432,7 +408,7 @@ constexpr uint32_t SPAN_BLOCK = SPAN_SCAN_THREADS * SPAN_PER_THREAD;   // chunk 
 // block index, which are resident or finished: CTAs are dispatched in index order) -> one carry word per chunk; the
 // thread that owns the document's last chunk writes the verdict (finish(), reference json_structural_indexer.mojo:147-186).
 // block_sum: 32 bytes per block, {count0, count1, flags, 0} then {generation, 0, 0, 0}.
-__global__ void __launch_bounds__(SJ_SCAN_THREADS) stage1_span_scan_kernel(const Stage1Params P, uint32_t nchunks) {
+__global__ void __launch_bounds__(SPAN_SCAN_THREADS) stage1_span_scan_kernel(const Stage1Params P, uint32_t nchunks) {
     __shared__ uint4 s_w[32];
     grid_dependency_wait();
     if (*reinterpret_cast<volatile uint32_t *>(P.spec_flag) == P.gen) return;

@@ -22,5 +22,5 @@ for kernel in os.environ.get('KERNELS', 'persistent,split').split(','):
         e1.record(); torch.cuda.synchronize()
         res = ctx.finish()
         ms = e0.elapsed_time(e1) / reps
-        print(os.environ.get('SJB200_LIB_VARIANT', 'default'), kernel, 'NW', nw, 'size_mib', size >> 20, 'ms %.4f' % ms, 'GB/s %.0f' % (size / ms / 1e6),
+        print(kernel, 'NW', nw, 'size_mib', size >> 20, 'ms %.4f' % ms, 'GB/s %.0f' % (size / ms / 1e6),
               'err', res.error, 'n', res.n, flush=True)
