@@ -4,9 +4,11 @@ nvcc cross-compiles without a GPU; the built .so files are git-ignored but trave
 """
 from __future__ import annotations
 
+import hashlib
 import os
 import subprocess
 import sys
+import tempfile
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
@@ -45,18 +47,35 @@ def build_synth(force: bool = False) -> str:
 
 def build_cpp_tests(force: bool = False) -> str:
     """tests/cpp/batch_test: the multi-GPU batch driver driven from C++ alone (links the product library, the workload
-    generator and -- as the checker -- the CPU oracle)."""
+    generator and -- as the checker -- the CPU oracle).  Returns the binary's path: in the tree, or in a temporary directory
+    when the tree is read-only and the in-tree binary is missing or older than its inputs."""
     root = os.path.dirname(PKG)
     src = os.path.join(root, "tests", "cpp", "batch_test.cpp")
     out = os.path.join(root, "tests", "cpp", "batch_test")
     oracle_dir = os.path.join(root, "oracle")
-    if force or _stale(out, [src, LIB, SYNTH_LIB]):
-        subprocess.check_call(["make", "-s", "-C", oracle_dir, "liboracle_stage1.so"])
-        nvcc = os.environ.get("NVCC", "nvcc")
-        subprocess.check_call([nvcc, "-O2", "-std=c++17", "-o", out, src, f"-L{PKG}", "-lsimdjson_b200", f"-L{os.path.dirname(SYNTH_LIB)}",
-                               "-lsjb200_synth", f"-L{oracle_dir}", "-loracle_stage1",
-                               "-Xlinker", "-rpath=$ORIGIN/../../mojo_simdjson_b200", "-Xlinker", "-rpath=$ORIGIN/../../mojo_simdjson_b200/synth",
-                               "-Xlinker", "-rpath=$ORIGIN/../../oracle", "-Wno-deprecated-gpu-targets"])
+    rpath = "$ORIGIN/../.."
+    if not (force or _stale(out, [src, LIB, SYNTH_LIB])):
+        return out
+    if not os.access(os.path.dirname(out), os.W_OK):
+        # a read-only checkout (tests run by a user who does not own the tree): build into a per-user temporary directory,
+        # named after the source and the tree it links against, with the tree's libraries found by absolute path
+        h = hashlib.sha1(root.encode())
+        with open(src, "rb") as f:
+            h.update(f.read())
+        d = os.path.join(tempfile.gettempdir(), f"sjb200-cpp-{os.getuid()}")
+        os.makedirs(d, mode=0o700, exist_ok=True)
+        out = os.path.join(d, f"batch_test-{h.hexdigest()[:16]}")
+        rpath = root
+        if not (force or _stale(out, [src, LIB, SYNTH_LIB])):
+            return out
+    subprocess.check_call(["make", "-s", "-C", oracle_dir, "liboracle_stage1.so"])
+    nvcc = os.environ.get("NVCC", "nvcc")
+    tmp = f"{out}.{os.getpid()}.tmp"   # concurrent builds each link their own, then rename atomically
+    subprocess.check_call([nvcc, "-O2", "-std=c++17", "-o", tmp, src, f"-L{PKG}", "-lsimdjson_b200", f"-L{os.path.dirname(SYNTH_LIB)}",
+                           "-lsjb200_synth", f"-L{oracle_dir}", "-loracle_stage1",
+                           "-Xlinker", f"-rpath={rpath}/mojo_simdjson_b200", "-Xlinker", f"-rpath={rpath}/mojo_simdjson_b200/synth",
+                           "-Xlinker", f"-rpath={rpath}/oracle", "-Wno-deprecated-gpu-targets"])
+    os.replace(tmp, out)
     return out
 
 

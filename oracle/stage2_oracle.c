@@ -328,7 +328,8 @@ EXPORT int32_t oracle_stage2_version(void) { return 1; }
  *   '}' / ']' | index of the matching start
  *   '"' | offset of the string's record in the string buffer
  *   'l' | 0 followed by the int64 value; 'd' | 0 followed by the IEEE-754 bits (parity UNPINNED for doubles, see (2) above:
- *                                 produced with strtod here and compared by the tests only where decimal -> binary is exact)
+ *                                 produced with strtod here, correctly rounded; the tests compare the kernel's
+ *                                 payloads with a restatement of its conversion, which is exact only on Clinger's fast path)
  *   't' 'f' 'n' | 0
  *   tape[N-1] = 'r' | 0
  * PARITY: error codes pinned by code reading; the reference's tests only assert SUCCESS on four fixtures.  Tape UNPINNED.
@@ -379,13 +380,13 @@ static int32_t walk_primitive(Walk *w, uint64_t i, int root) {
         const int32_t e = oracle_parse_number(w->buf, w->len, i, &isf, &v, &tl);
         if (e != SUCCESS) return e;
         if (isf) {
-            char tmp[512];
-            double d = 0.0;
-            if (tl < sizeof tmp) {
-                for (uint32_t k = 0; k < tl; k++) tmp[k] = (char)at(w->buf, w->len, i + k);
-                tmp[tl] = 0;
-                d = strtod(tmp, 0);
-            }
+            /* a float token can be arbitrarily long (digits and exponent have no length limit): copy it whole */
+            char *tmp = (char *)malloc((size_t)tl + 1);
+            if (!tmp) return CAPACITY_ERROR;
+            for (uint32_t k = 0; k < tl; k++) tmp[k] = (char)at(w->buf, w->len, i + k);
+            tmp[tl] = 0;
+            const double d = strtod(tmp, 0);
+            free(tmp);
             uint64_t bits;
             memcpy(&bits, &d, 8);
             tape_append(w, 0, 'd');

@@ -276,3 +276,19 @@ def test_walk_error_codes():
     # mixed: 99 arrays, then an object at depth 100 is fine, an array is not
     assert walk(b"[" * 99 + b'{"k":1}' + b"]" * 99).error == 0
     assert walk(b"[" * 99 + b"[1]" + b"]" * 99).error == D
+
+
+def test_walk_doubles_of_any_token_length():
+    """A float token has no length limit: the tape holds its correctly rounded value however long the token is."""
+    import struct
+
+    long = [b"5e" + b"0" * 600, b"1." + b"0" * 600, b"1" + b"2" * 599 + b".0", b"0." + b"0" * 600 + b"1", b"-" + b"9" * 600 + b".5",
+            b"1" * 600 + b"e-590"]
+    assert all(len(t) >= 600 for t in long)
+    toks = long + [b"1.5"] + [b"2.5e" + b"0" * (k - 5) + b"1" for k in (511, 512, 513)]   # 511 to 513 bytes
+    t = walk(b"[" + b",".join(toks) + b"]")
+    assert t.error == 0
+    m = len(toks)
+    assert t.tape.size == 2 * m + 4          # root, '[', a 'd' word and its payload per token, ']', root
+    assert [int(x) >> 56 for x in t.tape[2 : 2 + 2 * m : 2]] == [ord("d")] * m
+    assert [int(x) for x in t.tape[3 : 3 + 2 * m : 2]] ==[struct.unpack("<Q", struct.pack("<d", float(tok)))[0] for tok in toks]
