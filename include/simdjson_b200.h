@@ -174,13 +174,23 @@ int32_t sjb200_document_starts_device_async(sjb200_ctx *ctx, const uint8_t *d_by
                                             int32_t *d_scratch, uint64_t scratch_entries);
 
 /*
- * NDJSON / multi-document batches.  A batch is cut at '\n' into segments of at most seg_bytes (< 2^32) bytes;
- * every segment is an independent stage-1 call with segment-relative indexes, its own trailer and verdict --
- * exactly what the reference would produce if called once per segment.
+ * NDJSON / multi-document batches.  A batch is cut at '\n' into segments; every segment is an independent stage-1 call
+ * with segment-relative indexes, its own trailer and verdict -- exactly what the reference would produce if called once
+ * per segment.
+ *
+ * The cut rule (seg_bytes in [1, 2^31 - 1]): the batch has ncuts = ceil(len / seg_bytes) windows; cut k is the position
+ * right after the last '\n' among the bytes [k * seg_bytes, (k + 1) * seg_bytes), or len itself once
+ * (k + 1) * seg_bytes >= len.  Segments run from one cut to the next, so every segment but the last ends in '\n' and is
+ * at most 2 * seg_bytes - 1 bytes long.  A line longer than seg_bytes is accepted unless it leaves a whole window without
+ * a newline: with seg_bytes = 1000, a 1500-byte line at offset 500 becomes the segment [500, 2000), while a 1001-byte
+ * line at offset 0 is refused.  Blank lines are not skipped: a segment of nothing but newlines is indexed and reports
+ * EMPTY.  CAPACITY if seg_bytes is 0 or larger than 2^31 - 1, if ncuts > max_segments, or if a window other than the
+ * last holds no '\n'.
  *
  * sjb200_batch_split_device: finds the cut points of a device-resident batch.  seg_offsets must hold
- * max_segments + 1 entries; on return seg_offsets[0..*n_segments] are byte offsets (last one == len).
- * A line longer than seg_bytes -> CAPACITY.
+ * max_segments + 1 entries; on return seg_offsets[0..*n_segments] are byte offsets (last one == len).  The device
+ * splitter also refuses more than 4096 windows (CAPACITY).  sjb200_batch_split_host applies the same rule on the host,
+ * without that limit.
  */
 int32_t sjb200_batch_split_device(sjb200_ctx *ctx, const uint8_t *d_buf, uint64_t len, uint64_t seg_bytes,
                                   uint64_t *seg_offsets, uint32_t max_segments, uint32_t *n_segments);
@@ -207,7 +217,7 @@ int32_t sjb200_batch_run_device_async(sjb200_ctx *ctx, const uint8_t *d_buf, con
 
 /*
  * Multi-GPU batch driver (SURVEY.md section 8(b) / 8(e)): owns one context per GPU and the NCCL communicators.  The batch
- * is cut at '\n' into one shard per GPU and every shard into segments of at most ~seg_bytes (each segment = one reference
+ * is cut at '\n' into one shard per GPU and every shard into segments of < 2 * seg_bytes (the rule above; each segment = one reference
  * stage-1 call, dom_parser_implementation.mojo:65-69, on that byte range).  Per pass the GPUs exchange ONE NCCL all-gather
  * of the {error, n} rows of their segments -- the only inter-GPU traffic; the worst error is the maximum over the rows.
  * NCCL is loaded at run time (libnccl.so.2, or the path in SJB200_NCCL_LIB) and only when more than one GPU takes part.

@@ -1,7 +1,8 @@
 // batch_driver.cuh -- NDJSON / multi-document batch driver behind the C ABI (include/simdjson_b200.h, sjb200_batch_*).
 // Included at the end of capi.cu (it uses the context internals).
 //
-// A batch is cut at '\n' into shards (one per GPU) and every shard into segments of at most seg_bytes; a segment is
+// A batch is cut at '\n' into shards (one per GPU) and every shard into segments by the rule of sjb200_batch_split_host
+// (segments of up to 2 * seg_bytes - 1 bytes, each cut after the last newline of its seg_bytes window); a segment is
 // exactly one reference stage-1 call (segment-relative indexes, own trailer, own verdict: what
 // DomParserImplementation.stage1, include/generic/dom_parser_implementation.mojo:65-69, would return for that byte
 // range).  Bulk data never leaves its GPU.  The only inter-GPU traffic is ONE NCCL all-gather per pass of the

@@ -48,7 +48,7 @@ def test_host_splitter_without_gpu():
     assert cuts[0] == 0 and cuts[-1] == len(data)
     for a, b in zip(cuts, cuts[1:]):
         assert 0 < b - a <= 2000 and data[b - 1:b] == b"\n"
-    # a line longer than a segment cannot be cut
+    # a window without a newline cannot be cut
     rc = L.sjb200_batch_split_host(b"x" * 5000, 5000, 1000, offs, 63, C.byref(n))
     assert rc == errors.CAPACITY
 
