@@ -314,6 +314,52 @@ int32_t sjb200_stage2_tape_device_async(sjb200_ctx *ctx, const uint8_t *d_buf, u
 int32_t sjb200_stage2(sjb200_ctx *ctx, uint64_t *tape_out, uint64_t tape_capacity, uint8_t *strbuf_out, uint64_t strbuf_capacity,
                       uint64_t *tape_len, uint64_t *strbuf_len, uint64_t *inexact_doubles);
 
+/*
+ * Stage 2 over a stream of documents (NDJSON, or JSON documents simply concatenated), indexed by ONE stage-1 call: a
+ * verdict and a tape for every document, in one device pass.  Upstream simdjson calls this parse_many; the reference has
+ * no stream mode (generic/stage2/tape_builder.mojo:25 "TODO: add streaming").
+ *
+ * Documents.  Structural k starts a document iff the bracket depth over the structurals before it ('{' '[' +1, '}' ']' -1)
+ * is 0 -- the rule of sjb200_document_starts_device_async.  Document d is the tokens [doc_first[d], doc_first[d + 1]),
+ * doc_first[n_docs] = n.  Consequences: scalars separated by whitespace are separate documents (`1 2`, `"a" "b"`,
+ * `[1] 2` are two each); documents need no separator (`[1][2]`, `{}{}`); a document left unclosed swallows the rest of
+ * the stream; a stray close is a document of its own that fails, and everything after it up to where the depth returns
+ * to 0 belongs to it.  On well-formed input this separates documents the way parse_many does.  Lines play no part.
+ *
+ * Verdicts.  doc_status[d] is exactly the verdict the single-document walk (sjb200_stage2_tape_device_async, oracle
+ * oracle_stage2_walk) gives on document d alone, i.e. on its index sub-array followed by the trailer len, len, 0, in the
+ * same encoding: all ones = SUCCESS, else k << 16 | check << 8 | code with k relative to doc_first[d] (an unclosed last
+ * document fails at k = its length).  The reference's oddities hold per document: a root-level {} or [] is TAPE_ERROR,
+ * arrays hit DEPTH_ERROR one level before objects, more than 0xFFFFFF elements is CAPACITY.  A document's verdict never
+ * depends on any other document.
+ *
+ * Tape.  One tape for the stream; document d owns the words [doc_tape[d], doc_tape[d + 1]): 2 root words plus, per token,
+ * 1 word for strings, brackets and t f n, 2 for numbers, 0 for ':' ','.  The slice length does not depend on the verdict;
+ * the whole tape is at most 2 n + 2 n_docs <= 4 n words.  The slice of a successful document is the tape the
+ * single-document walk produces for it, with its root words and container indexes relative to the slice; its string words
+ * hold offsets into the stream's ONE string buffer, the one sjb200_stage2_primitives_device_async writes for all tokens in
+ * index order.  The words inside a failing document's slice are unspecified; nothing is written outside a document's slice.
+ *
+ * sjb200_stage2_stream_device_async: d_kind / d_err / d_value / d_str_off are the outputs of
+ * sjb200_stage2_primitives_device_async for the same indexes.  d_doc_first and d_doc_tape hold n + 1 entries, d_doc_status n
+ * (there are at most n documents); d_summary 4 x uint64: [0] documents, [1] failing documents, [2] tape words, [3] doubles
+ * not guaranteed exact.  Writes past tape_capacity are dropped; [2] still reports the full length.  EMPTY if n == 0,
+ * CAPACITY if len >= 2^32 or n >= 2^30.  Stream ordered on the context's stream; temporaries from its pool.
+ *
+ * sjb200_stage2_stream: host to host, after a successful sjb200_stage1 on this context (the resident copy, like
+ * sjb200_stage2).  doc_first and doc_tape hold max_docs + 1 entries, doc_status max_docs.  Returns the call's status, not
+ * the documents': SUCCESS when the outputs were delivered, also when documents fail (their verdicts are in doc_status);
+ * CAPACITY when n_docs > max_docs or the tape or the strings do not fit (nothing is copied, the sizes are set so that the
+ * caller can retry); UNINITIALIZED without such a stage-1 call.  Synchronous.
+ */
+int32_t sjb200_stage2_stream_device_async(sjb200_ctx *ctx, const uint8_t *d_buf, uint64_t len, const uint32_t *d_idx, uint64_t n,
+                                          const uint8_t *d_kind, const uint8_t *d_err, const int64_t *d_value, const uint64_t *d_str_off,
+                                          uint64_t *d_tape, uint64_t tape_capacity, uint32_t *d_doc_first, uint64_t *d_doc_tape,
+                                          uint64_t *d_doc_status, uint64_t *d_summary);
+int32_t sjb200_stage2_stream(sjb200_ctx *ctx, uint64_t *tape_out, uint64_t tape_capacity, uint8_t *strbuf_out, uint64_t strbuf_capacity,
+                             uint32_t *doc_first, uint64_t *doc_tape, uint64_t *doc_status, uint64_t max_docs, uint64_t *n_docs,
+                             uint64_t *n_failed, uint64_t *tape_len, uint64_t *strbuf_len, uint64_t *inexact_doubles);
+
 #ifdef __cplusplus
 }
 #endif

@@ -91,6 +91,16 @@ __device__ __forceinline__ Stk stk_concat(const Stk &a, const Stk &b) {
     }
     return r;
 }
+// Document streams: a document starts at every token of global bracket depth 0, and its walk must not see the stack of the
+// document before it (after a stray close that stack never empties again).  The scans then run over (flag, Stk) with
+// (fa, a) + (fb, b) = (fa | fb, fb ? b : a then b); the flag rides in the top bit of `pop`, which never reaches 2^30 (n < 2^30),
+// and stk_concat carries a's flag through unchanged when b has none.
+constexpr uint32_t STK_DOC_START = 0x80000000u;
+template <bool SEG>
+__device__ __forceinline__ Stk stk_combine(const Stk &a, const Stk &b) {
+    if (SEG && (b.pop & STK_DOC_START)) return b;
+    return stk_concat(a, b);
+}
 __device__ __forceinline__ Stk stk_shfl_up(const Stk &a, int d) {
     Stk r;
     r.pop = __shfl_up_sync(0xFFFFFFFFu, a.pop, d);
@@ -99,11 +109,12 @@ __device__ __forceinline__ Stk stk_shfl_up(const Stk &a, int d) {
     r.hi = __shfl_up_sync(0xFFFFFFFFu, a.hi, d);
     return r;
 }
+template <bool SEG>
 __device__ __forceinline__ Stk stk_warp_inclusive(Stk a, int lane) {
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
         const Stk o = stk_shfl_up(a, d);
-        if (lane >= d) a = stk_concat(o, a);
+        if (lane >= d) a = stk_combine<SEG>(o, a);
     }
     return a;
 }
@@ -111,21 +122,22 @@ __device__ __forceinline__ Stk stk_warp_inclusive(Stk a, int lane) {
 constexpr int TAPE_THREADS = 256, TAPE_PER_THREAD = 8, TAPE_BLOCK = TAPE_THREADS * TAPE_PER_THREAD;
 
 // inclusive scan over the CTA's 256 threads; returns this thread's EXCLUSIVE prefix inside the CTA, `total` = the CTA's
+template <bool SEG>
 __device__ __forceinline__ Stk stk_block_exclusive(const Stk mine, Stk *s_w /* [8] */, Stk &total) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const Stk incl = stk_warp_inclusive(mine, lane);
+    const Stk incl = stk_warp_inclusive<SEG>(mine, lane);
     if (lane == 31) s_w[warp] = incl;
     __syncthreads();
     Stk before = stk_identity(), all = stk_identity();
     for (int q = 0; q < TAPE_THREADS / 32; q++) {
-        if (q < warp) before = stk_concat(before, s_w[q]);
-        all = stk_concat(all, s_w[q]);
+        if (q < warp) before = stk_combine<SEG>(before, s_w[q]);
+        all = stk_combine<SEG>(all, s_w[q]);
     }
     total = all;
     __syncthreads();
     Stk prev = stk_shfl_up(incl, 1);            // the warp-inclusive value of the lane before = this lane's exclusive in-warp prefix
     if (lane == 0) prev = stk_identity();
-    return stk_concat(before, prev);
+    return stk_combine<SEG>(before, prev);
 }
 
 __device__ __forceinline__ uint8_t token_at(const uint8_t *buf, uint64_t len, const uint32_t *idx, uint64_t n, int64_t k) {
@@ -134,19 +146,29 @@ __device__ __forceinline__ uint8_t token_at(const uint8_t *buf, uint64_t len, co
     return s2_token(i < len ? (uint32_t)__ldg(buf + i) : 0x20u);
 }
 
+// the element of token k: stk_of(token), flagged where a document starts (stream mode only)
+template <bool STREAM>
+__device__ __forceinline__ Stk stk_elem(uint8_t t, const uint8_t *starts, uint64_t k) {
+    Stk e = stk_of(t);
+    if (STREAM && starts[k]) e.pop |= STK_DOC_START;
+    return e;
+}
+
+template <bool STREAM>
 __global__ void __launch_bounds__(TAPE_THREADS) tape_stack_totals_kernel(const uint8_t *__restrict__ buf, uint64_t len, const uint32_t *__restrict__ idx, uint64_t n,
-                                                                         Stk *__restrict__ block_total) {
+                                                                         Stk *__restrict__ block_total, const uint8_t *__restrict__ starts) {
     __shared__ Stk s_w[TAPE_THREADS / 32];
     const uint64_t k0 = (uint64_t)blockIdx.x * TAPE_BLOCK + (uint64_t)threadIdx.x * TAPE_PER_THREAD;
     Stk mine = stk_identity();
 #pragma unroll
     for (int j = 0; j < TAPE_PER_THREAD; j++)
-        if (k0 + j < n) mine = stk_concat(mine, stk_of(token_at(buf, len, idx, n, (int64_t)(k0 + j))));
+        if (k0 + j < n) mine = stk_combine<STREAM>(mine, stk_elem<STREAM>(token_at(buf, len, idx, n, (int64_t)(k0 + j)), starts, k0 + j));
     Stk total;
-    stk_block_exclusive(mine, s_w, total);
+    stk_block_exclusive<STREAM>(mine, s_w, total);
     if (threadIdx.x == 0) block_total[blockIdx.x] = total;
 }
 // one CTA: block_total[b] <- the stack operations of everything before block b (exclusive scan, in place)
+template <bool STREAM>
 __global__ void __launch_bounds__(1024) tape_stack_scan_kernel(Stk *block_total, uint32_t nblocks) {
     __shared__ Stk s_w[32];
     __shared__ Stk s_carry;
@@ -156,28 +178,42 @@ __global__ void __launch_bounds__(1024) tape_stack_scan_kernel(Stk *block_total,
     for (uint32_t b0 = 0; b0 < nblocks; b0 += 1024u) {
         const uint32_t b = b0 + threadIdx.x;
         const Stk v = b < nblocks ? block_total[b] : stk_identity();
-        const Stk incl = stk_warp_inclusive(v, lane);
+        const Stk incl = stk_warp_inclusive<STREAM>(v, lane);
         if (lane == 31) s_w[warp] = incl;
         __syncthreads();
         Stk before = s_carry;
-        for (int q = 0; q < warp; q++) before = stk_concat(before, s_w[q]);
+        for (int q = 0; q < warp; q++) before = stk_combine<STREAM>(before, s_w[q]);
         Stk prev = stk_shfl_up(incl, 1);
         if (lane == 0) prev = stk_identity();
-        const Stk excl = stk_concat(before, prev);
+        const Stk excl = stk_combine<STREAM>(before, prev);
         if (b < nblocks) block_total[b] = excl;
         __syncthreads();
-        if (threadIdx.x == 1023) s_carry = stk_concat(excl, v);
+        if (threadIdx.x == 1023) s_carry = stk_combine<STREAM>(excl, v);
         __syncthreads();
     }
 }
 
+// Stream mode (document streams): where documents start, the document of every token, the first token of every document
+// (doc_first[d], d <= n_docs, doc_first[n_docs] = n), where every document's tape slice starts, and one status word per document
+struct StreamArgs {
+    const uint8_t *starts;
+    const uint32_t *doc_of;
+    const uint32_t *doc_first;
+    const uint64_t *doc_tape;
+    unsigned long long *doc_status;
+};
+
 // per-token outputs of the grammar pass
 //   words[k]  tape words the token appends (0, 1, 2)
 //   cls[k]    multisplit class: 0 = none; else 1 + min(depth, 126), bit 7 set for commas (brackets: depth of the container's inside)
+// STREAM: every rule that reads the document's first token, second token, last token or length reads those of the token's own
+// document, the stack restarts empty at every document start, and errors go to the document's status word with the index
+// relative to its first token.
+template <bool STREAM>
 __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_t *__restrict__ buf, uint64_t len, const uint32_t *__restrict__ idx, uint64_t n,
                                                                     const uint8_t *__restrict__ prim_kind, const uint8_t *__restrict__ prim_err,
                                                                     const Stk *__restrict__ block_before, uint32_t *__restrict__ words, uint8_t *__restrict__ cls,
-                                                                    unsigned long long *__restrict__ first_err) {
+                                                                    unsigned long long *__restrict__ first_err, const StreamArgs sa) {
     __shared__ Stk s_w[TAPE_THREADS / 32];
     const uint64_t k0 = (uint64_t)blockIdx.x * TAPE_BLOCK + (uint64_t)threadIdx.x * TAPE_PER_THREAD;
     uint8_t tok[TAPE_PER_THREAD];
@@ -185,10 +221,11 @@ __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_
 #pragma unroll
     for (int j = 0; j < TAPE_PER_THREAD; j++) {
         tok[j] = token_at(buf, len, idx, n, (int64_t)(k0 + j));
-        if (k0 + j < n) mine = stk_concat(mine, stk_of(tok[j]));
+        if (k0 + j < n) mine = stk_combine<STREAM>(mine, stk_elem<STREAM>(tok[j], sa.starts, k0 + j));
     }
     Stk total;
-    Stk st = stk_concat(block_before[blockIdx.x], stk_block_exclusive(mine, s_w, total));   // the stack before this thread's first token
+    Stk st = stk_combine<STREAM>(block_before[blockIdx.x], stk_block_exclusive<STREAM>(mine, s_w, total));   // the stack before this thread's first token
+    if (STREAM) st.pop &= ~STK_DOC_START;
     uint8_t p1 = token_at(buf, len, idx, n, (int64_t)k0 - 1), p2 = token_at(buf, len, idx, n, (int64_t)k0 - 2);
     unsigned long long worst = ~0ull;
     const uint8_t first_tok = token_at(buf, len, idx, n, 0), last_tok = token_at(buf, len, idx, n, (int64_t)n - 1);
@@ -198,6 +235,19 @@ __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_
         if (k >= n) break;
         const uint8_t t = tok[j];
         const uint8_t nxt = (j + 1 < TAPE_PER_THREAD) ? tok[j + 1] : token_at(buf, len, idx, n, (int64_t)k + 1);
+        // the token's index in its document, the document's length, first and last token
+        uint64_t kl = k, nl = n;
+        uint8_t ft = first_tok, lt = last_tok;
+        uint32_t doc = 0;
+        if (STREAM) {
+            if (sa.starts[k]) st = stk_identity();
+            doc = sa.doc_of[k];
+            const uint32_t f = sa.doc_first[doc];
+            kl = k - f;
+            nl = (uint64_t)sa.doc_first[doc + 1] - f;
+            ft = kl == 1 ? p1 : TK_NONE;                                                  // only read at the second token
+            lt = kl == 0 ? token_at(buf, len, idx, n, (int64_t)(f + nl - 1)) : TK_NONE;   // only read at the first
+        }
         const bool underflow = st.pop != 0;
         const uint32_t depth = st.len;
         const int ctx = depth == 0 ? 0 : ((st.lo & 1ull) ? 2 : 1);   // 0 root, 1 object, 2 array
@@ -207,10 +257,10 @@ __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_
         if (underflow) {
             ok = false;
         } else if (ctx == 0) {
-            ok = (k == 0) && tk_value_start(t);                       // document_start: one value; anything after it is trailing content
-            if (k == 0 && ok) {
-                if (t == TK_LBRACE && last_tok != TK_RBRACE) ok = false;   // json_iterator.mojo:54-59
-                if (t == TK_LBRACK && last_tok != TK_RBRACK) ok = false;
+            ok = (kl == 0) && tk_value_start(t);                      // document_start: one value; anything after it is trailing content
+            if (kl == 0 && ok) {
+                if (t == TK_LBRACE && lt != TK_RBRACE) ok = false;         // json_iterator.mojo:54-59
+                if (t == TK_LBRACK && lt != TK_RBRACK) ok = false;
             }
         } else if (ctx == 2) {
             if (p1 == TK_LBRACK) ok = t == TK_RBRACK || tk_value_start(t);                 // array_begin / empty array
@@ -226,7 +276,7 @@ __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_
         }
         if (!ok) e = S2E_TAPE;
         // a root-level empty container is never consumed by the walk (json_iterator.mojo:61-65, 72-76): the index check at the end fails
-        if (!e && k == 1 && depth == 1 && tk_close(t) && n >= 2 && ((first_tok == TK_LBRACE && t == TK_RBRACE) || (first_tok == TK_LBRACK && t == TK_RBRACK))) e = S2E_TAPE;
+        if (!e && kl == 1 && depth == 1 && tk_close(t) && nl >= 2 && ((ft == TK_LBRACE && t == TK_RBRACE) || (ft == TK_LBRACK && t == TK_RBRACK))) e = S2E_TAPE;
         // ---- depth (object_begin / array_begin, not for empty containers)
         if (!e && tk_open(t)) {
             const bool empty = (t == TK_LBRACE && nxt == TK_RBRACE) || (t == TK_LBRACK && nxt == TK_RBRACK);
@@ -244,8 +294,9 @@ __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_
             prio = 2;
         }
         if (e) {
-            const unsigned long long cand = ((unsigned long long)k << 16) | ((unsigned long long)prio << 8) | e;
-            worst = cand < worst ? cand : worst;
+            const unsigned long long cand = ((unsigned long long)kl << 16) | ((unsigned long long)prio << 8) | e;
+            if (STREAM) atomicMin(sa.doc_status + doc, cand);   // a thread's tokens may belong to several documents
+            else worst = cand < worst ? cand : worst;
         }
         // ---- what the token appends, and its multisplit class
         uint32_t w = 0;
@@ -260,9 +311,11 @@ __global__ void __launch_bounds__(TAPE_THREADS) tape_grammar_kernel(const uint8_
         st = stk_concat(st, stk_of(t));
         p2 = p1;
         p1 = t;
+        // the walk of a document runs off its end with containers still open: TAPE_ERROR at the document's length
+        if (STREAM && kl + 1 == nl && st.pop == 0 && st.len != 0) atomicMin(sa.doc_status + doc, ((unsigned long long)nl << 16) | S2E_TAPE);
     }
     // the walk runs off the end with containers still open: the state that reads the trailer fails (TAPE_ERROR at index n)
-    if (k0 <= n - 1 && n - 1 < k0 + TAPE_PER_THREAD && st.pop == 0 && st.len != 0) {
+    if (!STREAM && k0 <= n - 1 && n - 1 < k0 + TAPE_PER_THREAD && st.pop == 0 && st.len != 0) {
         const unsigned long long cand = ((unsigned long long)n << 16) | S2E_TAPE;
         worst = cand < worst ? cand : worst;
     }
@@ -388,17 +441,26 @@ __device__ __forceinline__ uint64_t s2_double_bits(const DocBytes &at, uint64_t 
 }
 
 // summary[3]: number of doubles whose value is not guaranteed exact
+// STREAM: token k of document d writes at 1 + pos[k] + 2 d (two root words per document before it), and the tape indexes it
+// stores are relative to the start of its document's slice, doc_tape[d]
+template <bool STREAM>
 __global__ void __launch_bounds__(256) tape_emit_kernel(const uint8_t *__restrict__ buf, uint64_t len, const uint32_t *__restrict__ idx, uint64_t n,
                                                         const uint8_t *__restrict__ prim_kind, const int64_t *__restrict__ prim_value,
                                                         const uint64_t *__restrict__ str_off, const uint32_t *__restrict__ pos, const uint8_t *__restrict__ cls,
                                                         const uint32_t *__restrict__ slot_b, const uint32_t *__restrict__ rank_a, const uint32_t *__restrict__ sorted_b,
-                                                        uint32_t nbrackets, uint64_t *__restrict__ tape, uint64_t tape_cap, unsigned long long *__restrict__ summary) {
+                                                        uint32_t nbrackets, uint64_t *__restrict__ tape, uint64_t tape_cap, unsigned long long *__restrict__ summary,
+                                                        const StreamArgs sa) {
     const DocBytes at = {buf, len};
     for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t i = idx[k];
         const uint32_t ch = at(i);
         const uint8_t t = s2_token(ch);
-        const uint64_t p = 1ull + pos[k];             // word 0 is the root
+        uint32_t doc = 0, shift = 0;                  // STREAM: absolute position = slice-relative position + shift
+        if (STREAM && (tk_open(t) || tk_close(t))) {
+            doc = sa.doc_of[k];
+            shift = (uint32_t)sa.doc_tape[doc] - 2u * doc;
+        }
+        const uint64_t p = 1ull + pos[k] + (STREAM ? 2ull * sa.doc_of[k] : 0ull);   // word 0 is the root
         if (t == TK_STR) {
             if (p < tape_cap) tape[p] = ((uint64_t)'"' << 56) | str_off[k];
         } else if (t == TK_VAL) {
@@ -428,11 +490,14 @@ __global__ void __launch_bounds__(256) tape_emit_kernel(const uint8_t *__restric
                 const uint32_t ko = open ? (uint32_t)k : o, kc = open ? o : (uint32_t)k;
                 if (open) {
                     const uint64_t count = (kc == ko + 1u) ? 0ull : (uint64_t)(rank_a[kc] - rank_a[ko] - 1u) + 1ull;
-                    if (p < tape_cap) tape[p] = ((uint64_t)ch << 56) | ((count & 0xFFFFFFull) << 32) | (uint64_t)(1u + pos[kc] + 1u);
+                    if (p < tape_cap) tape[p] = ((uint64_t)ch << 56) | ((count & 0xFFFFFFull) << 32) | (uint64_t)(1u + pos[kc] + 1u - shift);
                 } else {
                     const uint64_t count = (kc == ko + 1u) ? 0ull : (uint64_t)(rank_a[kc] - rank_a[ko] - 1u) + 1ull;
-                    if (count > 0xFFFFFFull) atomicMin(summary, ((unsigned long long)k << 16) | (3ull << 8) | S2E_CAPACITY);   // tape_builder.mojo:239-241
-                    if (p < tape_cap) tape[p] = ((uint64_t)ch << 56) | (uint64_t)(1u + pos[ko]);
+                    if (count > 0xFFFFFFull) {   // tape_builder.mojo:239-241
+                        if (STREAM) atomicMin(sa.doc_status + doc, ((unsigned long long)(k - sa.doc_first[doc]) << 16) | (3ull << 8) | S2E_CAPACITY);
+                        else atomicMin(summary, ((unsigned long long)k << 16) | (3ull << 8) | S2E_CAPACITY);
+                    }
+                    if (p < tape_cap) tape[p] = ((uint64_t)ch << 56) | (uint64_t)(1u + pos[ko] - shift);
                 }
             }
         }
@@ -443,6 +508,54 @@ __global__ void tape_roots_kernel(uint64_t *tape, uint64_t tape_cap, const unsig
     if (0 < tape_cap) tape[0] = ((uint64_t)'r' << 56) | N;
     if (N - 1 < tape_cap) tape[N - 1] = (uint64_t)'r' << 56;
     summary[2] = N;
+}
+
+// ---- document streams ----
+// flags[k] = starts[k] (the exclusive scan of flags then numbers the documents)
+__global__ void __launch_bounds__(256) stream_flags_kernel(const uint8_t *__restrict__ starts, uint64_t n, uint32_t *__restrict__ flags) {
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (uint64_t)gridDim.x * blockDim.x) flags[k] = starts[k];
+}
+// doc_of[k] (in place over the scanned flags) and doc_first[d]; doc_first[n_docs] = n
+__global__ void __launch_bounds__(256) stream_docs_kernel(const uint8_t *__restrict__ starts, uint64_t n, uint32_t *__restrict__ doc_of,
+                                                          uint32_t *__restrict__ doc_first, const unsigned long long *__restrict__ n_docs) {
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t before = doc_of[k];
+        if (starts[k]) {
+            doc_first[before] = (uint32_t)k;
+            doc_of[k] = before;
+        } else {
+            doc_of[k] = before - 1u;
+        }
+        if (k == 0) doc_first[*n_docs] = (uint32_t)n;
+    }
+}
+// doc_tape[d] = words of the tokens before document d + its 2 d root words before it; both root words of every document;
+// summary[2] = the whole tape's length
+__global__ void __launch_bounds__(256) stream_roots_kernel(const uint32_t *__restrict__ doc_first, const uint32_t *__restrict__ pos, uint64_t n,
+                                                           const unsigned long long *__restrict__ n_docs, const unsigned long long *__restrict__ total_words,
+                                                           uint64_t *__restrict__ doc_tape, uint64_t *__restrict__ tape, uint64_t tape_cap,
+                                                           unsigned long long *__restrict__ summary) {
+    const uint64_t nd = *n_docs, N = *total_words + 2ull * nd;
+    for (uint64_t d = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; d < nd; d += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t off = (uint64_t)pos[doc_first[d]] + 2ull * d;
+        const uint64_t end = d + 1 < nd ? (uint64_t)pos[doc_first[d + 1]] + 2ull * (d + 1) : N;
+        doc_tape[d] = off;
+        if (off < tape_cap) tape[off] = ((uint64_t)'r' << 56) | (end - off);
+        if (end - 1 < tape_cap) tape[end - 1] = (uint64_t)'r' << 56;
+        if (d == 0) {
+            doc_tape[nd] = N;
+            summary[2] = N;
+        }
+    }
+}
+// summary[1] = documents whose status is not SUCCESS
+__global__ void __launch_bounds__(256) stream_failed_kernel(const unsigned long long *__restrict__ doc_status, unsigned long long *__restrict__ summary) {
+    const uint64_t nd = summary[0];
+    for (uint64_t d0 = (uint64_t)blockIdx.x * blockDim.x; d0 < nd; d0 += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t d = d0 + threadIdx.x;
+        const int c = __syncthreads_count(d < nd && doc_status[d] != ~0ull);
+        if (threadIdx.x == 0 && c) atomicAdd(summary + 1, (unsigned long long)c);
+    }
 }
 
 // ---- exclusive prefix sum of uint32 (in place), same three launches as the uint64 one of stage2_primitives.cuh ----
@@ -555,9 +668,9 @@ int32_t sjb200_stage2_tape_device_async(sjb200_ctx *c, const uint8_t *d_buf, uin
         return SJB200_MEMALLOC;
     }
     // depth / container type: the bit-stack scan; then the grammar, the words and the multisplit classes
-    tape_stack_totals_kernel<<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_stk);
-    tape_stack_scan_kernel<<<1, 1024, 0, s>>>(d_stk, (uint32_t)nblk);
-    tape_grammar_kernel<<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_stk, d_words, d_cls, summary);
+    tape_stack_totals_kernel<false><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_stk, nullptr);
+    tape_stack_scan_kernel<false><<<1, 1024, 0, s>>>(d_stk, (uint32_t)nblk);
+    tape_grammar_kernel<false><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_stk, d_words, d_cls, summary, StreamArgs{});
     // where every token's words go
     e = scan32_exclusive(d_words, n, summary + 1, c->pool, s);
     // brackets and commas by depth: two class-major histograms, each scanned on its own, then the ranks
@@ -570,14 +683,182 @@ int32_t sjb200_stage2_tape_device_async(sjb200_ctx *c, const uint8_t *d_buf, uin
     if (e == cudaSuccess) {
         tape_multisplit_rank_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist, 0u, d_slot, d_rank, d_sorted);
         const unsigned grid = (unsigned)((n + 255) / 256 < (uint64_t)c->sm_count * 32 ? (n + 255) / 256 : (uint64_t)c->sm_count * 32);
-        tape_emit_kernel<<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_value, d_str_off, d_words, d_cls, d_slot, d_rank, d_sorted, nbrackets_upper, d_tape,
-                                              tape_capacity, summary);
+        tape_emit_kernel<false><<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_value, d_str_off, d_words, d_cls, d_slot, d_rank, d_sorted, nbrackets_upper,
+                                                     d_tape, tape_capacity, summary, StreamArgs{});
         tape_roots_kernel<<<1, 1, 0, s>>>(d_tape, tape_capacity, summary + 1, summary);
         e = cudaGetLastError();
     }
     release();
     c->launches += 14;
     return e == cudaSuccess ? SJB200_SUCCESS : cuda_err(e);
+}
+
+// Stage 2 over a stream of documents (include/simdjson_b200.h): the same launches as the single-document walk, on the
+// segmented stack scan, plus the document split (structural bytes and the depth scan of sjb200_document_starts_device_async),
+// the document numbering, the roots of every slice and the count of failing documents.
+int32_t sjb200_stage2_stream_device_async(sjb200_ctx *c, const uint8_t *d_buf, uint64_t len, const uint32_t *d_idx, uint64_t n, const uint8_t *d_kind,
+                                          const uint8_t *d_err, const int64_t *d_value, const uint64_t *d_str_off, uint64_t *d_tape, uint64_t tape_capacity,
+                                          uint32_t *d_doc_first, uint64_t *d_doc_tape, uint64_t *d_doc_status, uint64_t *d_summary) {
+    if (!c) return SJB200_UNINITIALIZED;
+    if (!d_buf || !d_idx || !d_kind || !d_err || !d_value || !d_str_off || !d_tape || !d_doc_first || !d_doc_tape || !d_doc_status || !d_summary)
+        return SJB200_UNINITIALIZED;
+    if (len > 0xFFFFFFFFull || n >= (1ull << 30)) return SJB200_CAPACITY;   // tape positions are 32 bit: up to 4 n words
+    if (n == 0) return SJB200_EMPTY;
+    CK(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    unsigned long long *summary = reinterpret_cast<unsigned long long *>(d_summary);
+    unsigned long long *doc_status = reinterpret_cast<unsigned long long *>(d_doc_status);
+    // summary: [0] documents, [1] failing documents, [2] tape length, [3] inexact doubles
+    CK(cudaMemsetAsync(d_summary, 0, 32, s));
+    CK(cudaMemsetAsync(d_doc_status, 0xFF, n * 8, s));
+    const uint64_t nblk = (n + TAPE_BLOCK - 1) / TAPE_BLOCK;
+    const uint64_t dblk = (n + DEPTH_BLOCK - 1) / DEPTH_BLOCK;
+    const uint32_t ntiles = (uint32_t)((n + MS_TILE - 1) / MS_TILE);
+    const size_t hist_entries = (size_t)2 * MS_CLASSES * ntiles;
+    Stk *d_stk = nullptr;
+    uint32_t *d_words = nullptr, *d_slot = nullptr, *d_rank = nullptr, *d_sorted = nullptr, *d_hist = nullptr, *d_doc = nullptr;
+    uint8_t *d_cls = nullptr, *d_bytes = nullptr, *d_starts = nullptr;
+    int32_t *d_depth = nullptr;
+    unsigned long long *d_tot = nullptr;
+    cudaError_t e = cudaMallocFromPoolAsync(&d_stk, nblk * sizeof(Stk), c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_words, n * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_cls, n, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_slot, n * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_rank, n * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sorted, n * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_hist, hist_entries * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tot, 32, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_doc, n * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_bytes, n, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_starts, n, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_depth, dblk * 4, c->pool, s);
+    auto release = [&]() {
+        if (d_stk) cudaFreeAsync(d_stk, s);
+        if (d_words) cudaFreeAsync(d_words, s);
+        if (d_cls) cudaFreeAsync(d_cls, s);
+        if (d_slot) cudaFreeAsync(d_slot, s);
+        if (d_rank) cudaFreeAsync(d_rank, s);
+        if (d_sorted) cudaFreeAsync(d_sorted, s);
+        if (d_hist) cudaFreeAsync(d_hist, s);
+        if (d_tot) cudaFreeAsync(d_tot, s);
+        if (d_doc) cudaFreeAsync(d_doc, s);
+        if (d_bytes) cudaFreeAsync(d_bytes, s);
+        if (d_starts) cudaFreeAsync(d_starts, s);
+        if (d_depth) cudaFreeAsync(d_depth, s);
+    };
+    if (e != cudaSuccess) {
+        release();
+        cudaGetLastError();
+        return SJB200_MEMALLOC;
+    }
+    const unsigned grid = (unsigned)((n + 255) / 256 < (uint64_t)c->sm_count * 32 ? (n + 255) / 256 : (uint64_t)c->sm_count * 32);
+    // where documents start: the bracket depth over the structural bytes
+    int32_t rc = sjb200_structural_bytes_device_async(c, d_buf, len, d_idx, n, d_bytes);
+    if (rc == SJB200_SUCCESS) rc = sjb200_document_starts_device_async(c, d_bytes, n, d_starts, d_depth, dblk);
+    if (rc != SJB200_SUCCESS) {
+        release();
+        return rc;
+    }
+    // the document of every token, and the first token of every document
+    stream_flags_kernel<<<grid, 256, 0, s>>>(d_starts, n, d_doc);
+    e = scan32_exclusive(d_doc, n, summary, c->pool, s);
+    if (e == cudaSuccess) stream_docs_kernel<<<grid, 256, 0, s>>>(d_starts, n, d_doc, d_doc_first, summary);
+    const StreamArgs sa{d_starts, d_doc, d_doc_first, d_doc_tape, doc_status};
+    // depth / container type inside each document: the segmented bit-stack scan; then the grammar, the words and the classes
+    if (e == cudaSuccess) {
+        tape_stack_totals_kernel<true><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_stk, d_starts);
+        tape_stack_scan_kernel<true><<<1, 1024, 0, s>>>(d_stk, (uint32_t)nblk);
+        tape_grammar_kernel<true><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_stk, d_words, d_cls, nullptr, sa);
+        e = scan32_exclusive(d_words, n, d_tot + 2, c->pool, s);
+    }
+    if (e == cudaSuccess) {
+        stream_roots_kernel<<<grid, 256, 0, s>>>(d_doc_first, d_words, n, summary, d_tot + 2, d_doc_tape, d_tape, tape_capacity, summary);
+        tape_multisplit_hist_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist);
+        e = scan32_exclusive(d_hist, (uint64_t)MS_CLASSES * ntiles, d_tot, c->pool, s);
+    }
+    if (e == cudaSuccess) e = scan32_exclusive(d_hist + (size_t)MS_CLASSES * ntiles, (uint64_t)MS_CLASSES * ntiles, d_tot + 1, c->pool, s);
+    if (e == cudaSuccess) {
+        tape_multisplit_rank_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist, 0u, d_slot, d_rank, d_sorted);
+        tape_emit_kernel<true><<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_value, d_str_off, d_words, d_cls, d_slot, d_rank, d_sorted, (uint32_t)n, d_tape,
+                                                    tape_capacity, summary, sa);
+        stream_failed_kernel<<<grid, 256, 0, s>>>(doc_status, summary);
+        e = cudaGetLastError();
+    }
+    release();
+    c->launches += 22;   // and 4 in the document split
+    return e == cudaSuccess ? SJB200_SUCCESS : cuda_err(e);
+}
+
+// Host-to-host stage 2 over a stream of documents: sjb200_stage2's counterpart for NDJSON and concatenated JSON.
+int32_t sjb200_stage2_stream(sjb200_ctx *c, uint64_t *tape_out, uint64_t tape_capacity, uint8_t *strbuf_out, uint64_t strbuf_capacity, uint32_t *doc_first,
+                             uint64_t *doc_tape, uint64_t *doc_status, uint64_t max_docs, uint64_t *n_docs, uint64_t *n_failed, uint64_t *tape_len,
+                             uint64_t *strbuf_len, uint64_t *inexact_doubles) {
+    if (!c || !tape_out || !strbuf_out || !doc_first || !doc_tape || !doc_status) return SJB200_UNINITIALIZED;
+    if (c->resident_len == 0 || c->resident_n == 0) return SJB200_UNINITIALIZED;   // no successful stage 1 before this call
+    const uint64_t len = c->resident_len, n = c->resident_n;
+    CK(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    const uint64_t sb_cap = len + 2 * n + 64, tp_cap = 4 * n;
+    uint8_t *d_kind = nullptr, *d_err = nullptr, *d_sb = nullptr;
+    int64_t *d_val = nullptr;
+    uint64_t *d_off = nullptr, *d_tape = nullptr, *d_sum = nullptr, *d_dtape = nullptr, *d_dstatus = nullptr;
+    uint32_t *d_dfirst = nullptr;
+    cudaError_t e = cudaMallocFromPoolAsync(&d_kind, n, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_err, n, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_val, n * 8, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_off, n * 8, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sb, sb_cap, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tape, tp_cap * 8, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sum, 64, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dfirst, (n + 1) * 4, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dtape, (n + 1) * 8, c->pool, s);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dstatus, n * 8, c->pool, s);
+    auto release = [&]() {
+        if (d_kind) cudaFreeAsync(d_kind, s);
+        if (d_err) cudaFreeAsync(d_err, s);
+        if (d_val) cudaFreeAsync(d_val, s);
+        if (d_off) cudaFreeAsync(d_off, s);
+        if (d_sb) cudaFreeAsync(d_sb, s);
+        if (d_tape) cudaFreeAsync(d_tape, s);
+        if (d_sum) cudaFreeAsync(d_sum, s);
+        if (d_dfirst) cudaFreeAsync(d_dfirst, s);
+        if (d_dtape) cudaFreeAsync(d_dtape, s);
+        if (d_dstatus) cudaFreeAsync(d_dstatus, s);
+    };
+    if (e != cudaSuccess) {
+        release();
+        cudaGetLastError();
+        return SJB200_MEMALLOC;
+    }
+    int32_t rc = sjb200_stage2_primitives_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_sb, sb_cap, d_sum);
+    if (rc == SJB200_SUCCESS)
+        rc = sjb200_stage2_stream_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_tape, tp_cap, d_dfirst, d_dtape, d_dstatus, d_sum + 4);
+    uint64_t sum[8] = {};
+    if (rc == SJB200_SUCCESS) {
+        e = cudaMemcpyAsync(sum, d_sum, 64, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) rc = cuda_err(e);
+    }
+    if (rc == SJB200_SUCCESS) {
+        const uint64_t sb = sum[1], nd = sum[4], tl = sum[6];
+        if (n_docs) *n_docs = nd;
+        if (n_failed) *n_failed = sum[5];
+        if (tape_len) *tape_len = tl;
+        if (strbuf_len) *strbuf_len = sb;
+        if (inexact_doubles) *inexact_doubles = sum[7];
+        if (nd > max_docs || tl > tape_capacity || sb > strbuf_capacity) rc = SJB200_CAPACITY;
+        if (rc == SJB200_SUCCESS) {
+            e = cudaMemcpyAsync(tape_out, d_tape, tl * 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess && sb) e = cudaMemcpyAsync(strbuf_out, d_sb, sb, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(doc_first, d_dfirst, (nd + 1) * 4, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(doc_tape, d_dtape, (nd + 1) * 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(doc_status, d_dstatus, nd * 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+            if (e != cudaSuccess) rc = cuda_err(e);
+        }
+    }
+    release();
+    return rc;
 }
 
 // Host-to-host stage 2, the drop-in for DomParserImplementation.stage2 (include/generic/dom_parser_implementation.mojo:71-83):

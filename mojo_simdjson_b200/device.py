@@ -165,6 +165,28 @@ class Stage1Context:
             raise RuntimeError(f"stage-2 tape failed: {errors.NAMES.get(rc, rc)}")
         return tape, summary
 
+    def stage2_stream(self, buf: torch.Tensor, idx: torch.Tensor, n: int, prims: dict, tape_capacity: int | None = None):
+        """Stage 2 over a stream of documents (NDJSON or concatenated JSON; include/simdjson_b200.h,
+        sjb200_stage2_stream_device_async): one verdict and one tape slice per document.  `prims` = the result of
+        stage2_primitives for the same indexes; its string buffer is the one the string words point into.  Returns a dict of
+        device tensors: tape (int64, 4 n words unless tape_capacity is given), doc_first (int32 [n_docs + 1]), doc_tape
+        (int64 [n_docs + 1]), doc_status (int64 [n_docs], -1 = SUCCESS), summary (int64 [4]: documents, failing documents,
+        tape length, inexact doubles).  Synchronises to learn n_docs."""
+        dev = buf.device
+        tape = torch.zeros(4 * n if tape_capacity is None else max(tape_capacity, 1), dtype=torch.int64, device=dev)
+        first = torch.empty(n + 1, dtype=torch.int32, device=dev)
+        doc_tape = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        status = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+        summary = torch.empty(4, dtype=torch.int64, device=dev)
+        rc = self._lib.sjb200_stage2_stream_device_async(self._ctx, buf.data_ptr(), buf.numel(), idx.data_ptr(), n, prims["kind"].data_ptr(),
+                                                         prims["error"].data_ptr(), prims["value"].data_ptr(), prims["str_off"].data_ptr(),
+                                                         tape.data_ptr(), tape.numel() if tape_capacity is None else tape_capacity,
+                                                         first.data_ptr(), doc_tape.data_ptr(), status.data_ptr(), summary.data_ptr())
+        if rc != errors.SUCCESS:
+            raise RuntimeError(f"stage-2 stream walk failed: {errors.NAMES.get(rc, rc)}")
+        nd = int(summary[0].item())
+        return {"tape": tape, "doc_first": first[: nd + 1], "doc_tape": doc_tape[: nd + 1], "doc_status": status[:nd], "summary": summary}
+
     def last_elapsed_ms(self) -> float:
         return float(self._lib.sjb200_last_elapsed_ms(self._ctx))
 

@@ -65,6 +65,35 @@ class Document:
         return "\n".join(out) + "\n", True
 
 
+class DocumentStream:
+    """The documents of one stream (NDJSON or concatenated JSON) after DomParserImplementation.stage2_stream(): one tape with
+    a slice per document, one string buffer, one verdict per document (include/simdjson_b200.h, sjb200_stage2_stream)."""
+
+    def __init__(self, tape, string_buf, doc_first, doc_tape, doc_status, n_failed: int, inexact_doubles: int):
+        self.tape = tape                    # uint64, every document's slice back to back
+        self.string_buf = string_buf        # uint8, the records every slice's string words point into
+        self.doc_first = doc_first          # uint32 [len + 1]: first structural of every document
+        self.doc_tape = doc_tape            # uint64 [len + 1]: where every document's slice starts
+        self.doc_status = doc_status        # uint64 [len]: all ones = SUCCESS, else k << 16 | check << 8 | code
+        self.n_failed = n_failed
+        self.inexact_doubles = inexact_doubles
+
+    def __len__(self) -> int:
+        return int(self.doc_status.size)
+
+    def error(self, d: int) -> int:
+        """The error code of document d (0 = SUCCESS)."""
+        s = int(self.doc_status[d])
+        return 0 if s == (1 << 64) - 1 else s & 0xFF
+
+    def document(self, d: int) -> Document:
+        """Document d as a Document: a view of its tape slice and the stream's string buffer.  Meaningful when error(d) == 0."""
+        doc = Document()
+        doc.tape = self.tape[int(self.doc_tape[d]) : int(self.doc_tape[d + 1])]
+        doc.string_buf = self.string_buf
+        return doc
+
+
 class DomParserImplementation:
     """Stage-1 half of the reference's DomParserImplementation, backed by the B200 kernel."""
 
@@ -78,6 +107,7 @@ class DomParserImplementation:
         self.structural_indexes = np.zeros(0, dtype=np.uint32)
         self.next_structural_index = 0
         self.document = Document()
+        self.stream: DocumentStream | None = None    # stage2_stream()'s result
         self.utf8_error = 0                          # not in the reference: its Utf8Checker is a stub
         self._capacity = 0
         self._max_depth = 100
@@ -153,4 +183,24 @@ class DomParserImplementation:
             self.document.tape = tape[: tl.value]
             self.document.string_buf = sbuf[: sl.value]
             self.document.inexact_doubles = int(inexact.value)
+        return rc
+
+    def stage2_stream(self) -> int:
+        """Stage 2 over a stream of documents (NDJSON or concatenated JSON) that stage1() indexed: one verdict and one tape
+        slice per document, in `self.stream` (a DocumentStream).  Returns the call's code: SUCCESS when the outputs were
+        delivered, also when documents fail; the documents' verdicts are in self.stream."""
+        n, length = int(self.n_structural_indexes), int(self.length)
+        if self.buf is None or n == 0:
+            return errors.UNINITIALIZED
+        tape = np.zeros(4 * n, dtype=np.uint64)
+        sbuf = np.zeros(length + 2 * n + 64, dtype=np.uint8)
+        first = np.zeros(n + 1, dtype=np.uint32)
+        doc_tape = np.zeros(n + 1, dtype=np.uint64)
+        status = np.zeros(n, dtype=np.uint64)
+        nd, nf, tl, sl, inexact = (C.c_uint64(0) for _ in range(5))
+        rc = self._lib.sjb200_stage2_stream(self._ctx, tape.ctypes.data, tape.size, sbuf.ctypes.data, sbuf.size, first.ctypes.data, doc_tape.ctypes.data,
+                                            status.ctypes.data, n, C.byref(nd), C.byref(nf), C.byref(tl), C.byref(sl), C.byref(inexact))
+        if rc == errors.SUCCESS:
+            d = int(nd.value)
+            self.stream = DocumentStream(tape[: tl.value], sbuf[: sl.value], first[: d + 1], doc_tape[: d + 1], status[:d], int(nf.value), int(inexact.value))
         return rc
