@@ -52,6 +52,12 @@ extern "C" {
 #define SJB200_UNESCAPED_CHARS 14
 #define SJB200_UNCLOSED_STRING 15
 #define SJB200_UNEXPECTED_ERROR 24
+/* codes of the JSON Pointer lookups (sjb200_at_pointers_device_async) */
+#define SJB200_TAPE_ERROR 3
+#define SJB200_INCORRECT_TYPE 17
+#define SJB200_INDEX_OUT_OF_BOUNDS 19
+#define SJB200_NO_SUCH_FIELD 20
+#define SJB200_INVALID_JSON_POINTER 22
 
 /* flags */
 #define SJB200_FLAG_VALIDATE_UTF8 1u /* return UTF8_ERROR (lowest priority) when the input is not valid UTF-8 */
@@ -359,6 +365,62 @@ int32_t sjb200_stage2_stream_device_async(sjb200_ctx *ctx, const uint8_t *d_buf,
 int32_t sjb200_stage2_stream(sjb200_ctx *ctx, uint64_t *tape_out, uint64_t tape_capacity, uint8_t *strbuf_out, uint64_t strbuf_capacity,
                              uint32_t *doc_first, uint64_t *doc_tape, uint64_t *doc_status, uint64_t max_docs, uint64_t *n_docs,
                              uint64_t *n_failed, uint64_t *tape_len, uint64_t *strbuf_len, uint64_t *inexact_doubles);
+
+/*
+ * JSON Pointer (RFC 6901) lookups on the device tapes: for K pointers and D documents, K columns of D cells.  The rules
+ * below are this project's definition (restated in tests/pointer_oracle.py, DESIGN.md section 7.2).  They follow upstream
+ * simdjson's DOM element::at_pointer on well-formed pointers; where upstream releases differ (a token applied to a scalar)
+ * this table pins the choice.
+ *
+ * Input: a tape with one slice per document, its string buffer, each document's slice bounds doc_tape[d] .. doc_tape[d + 1]
+ * and status word doc_status[d] -- the outputs of sjb200_stage2_stream_device_async.  One document from
+ * sjb200_stage2_tape_device_async is the case D = 1: doc_tape = {0, summary[2]}, doc_status = {summary[0]}.
+ *
+ * Pointers.  Pointer k is the bytes pointers[pointer_offsets[k] .. pointer_offsets[k + 1]) (UTF-8 by convention).  It is
+ * empty (the root value, slice word 1) or a sequence of '/'-prefixed tokens; in a token "~1" becomes '/' and "~0" becomes
+ * '~', left to right ("~01" is "~1").  A pointer that is not empty and does not start with '/' ("#/..." URI fragments
+ * included), a '~' not followed by '0' or '1', or decreasing offsets: INVALID_JSON_POINTER for the whole call, nothing
+ * written.  More than SJB200_POINTER_MAX_COUNT pointers or more than SJB200_POINTER_MAX_BYTES pointer bytes in all: CAPACITY.
+ *
+ * Cells.  The walk starts at the root value and applies one token at a time:
+ *   object     the FIRST member in tape order whose unescaped key bytes equal the token's (upstream's DOM at_key; python's
+ *              json keeps the last); none: NO_SUCH_FIELD
+ *   array      of c elements (exact: a successful document has none of 2^24 or more), checked in this order:
+ *              token "-": INDEX_OUT_OF_BOUNDS; empty token: INVALID_JSON_POINTER; a byte outside 0-9: INCORRECT_TYPE ("0a");
+ *              more than one digit with a leading 0: INVALID_JSON_POINTER; value >= c (saturating, no overflow):
+ *              INDEX_OUT_OF_BOUNDS; else element value
+ *   scalar     a token left: NO_SUCH_FIELD
+ * A failing document (status not all ones) gives every cell its own code status & 0xFF; its slice is never read.
+ * Guards against caller-supplied arrays (a tape this library writes never triggers them): a slice that reaches past
+ * tape_len, or a string record the walk reads that reaches past strbuf_len: CAPACITY; a tape word that points outside the
+ * slice or its container, or a word of the wrong type: TAPE_ERROR.  Every read stays inside the slice and strbuf_len.
+ *
+ * Outputs, pointer-major ([K][D], cell k * n_docs + d; each column contiguous):
+ *   type   uint8: the tape type character of the value found ('{' '[' '"' 'l' 'd' 't' 'f' 'n'), 0 when code != SUCCESS
+ *   code   uint8: SUCCESS, or the code from the rules above
+ *   value  int64: 'l' the integer; 'd' the IEEE-754 bits (the tape's payload, with its inexactness caveat); 't' 1, 'f' 'n' 0;
+ *          '"' the offset of the string's {uint32 length, bytes} record in the string buffer; '{' '[' the slice-relative
+ *          index of the container's open word.  0 when code != SUCCESS.
+ * Cost: a cell costs O(members or elements skipped); element i of one array costs about i dependent loads.
+ *
+ * sjb200_at_pointers_device_async: pointers and pointer_offsets (K + 1 entries) are host memory, everything else device
+ * memory.  Stream ordered on the context's stream.  n_docs == 0 or K == 0: SUCCESS, nothing written.  Nothing is written
+ * outside the K x D cells.
+ *
+ * sjb200_stage2_stream_at_pointers: host to host, over the document the preceding successful sjb200_stage1 on this context
+ * left resident (like sjb200_stage2_stream): the primitives, the stream walk and the lookups run on the device; only the
+ * K x D cells come back, plus the string buffer if strbuf_out is not NULL (to read string cells).  cells_capacity is in
+ * cells.  CAPACITY when the cells or the strings do not fit (nothing copied; *n_docs and *strbuf_len are set so that the
+ * caller can retry); UNINITIALIZED without such a stage-1 call.  Synchronous.
+ */
+#define SJB200_POINTER_MAX_COUNT 1024
+#define SJB200_POINTER_MAX_BYTES 16384
+int32_t sjb200_at_pointers_device_async(sjb200_ctx *ctx, const uint64_t *d_tape, uint64_t tape_len, const uint8_t *d_strbuf, uint64_t strbuf_len,
+                                        const uint64_t *d_doc_tape, const uint64_t *d_doc_status, uint64_t n_docs, const uint8_t *pointers,
+                                        const uint64_t *pointer_offsets, uint64_t n_pointers, uint8_t *d_type, uint8_t *d_code, int64_t *d_value);
+int32_t sjb200_stage2_stream_at_pointers(sjb200_ctx *ctx, const uint8_t *pointers, const uint64_t *pointer_offsets, uint64_t n_pointers,
+                                         uint8_t *type_out, uint8_t *code_out, int64_t *value_out, uint64_t cells_capacity, uint8_t *strbuf_out,
+                                         uint64_t strbuf_capacity, uint64_t *n_docs, uint64_t *strbuf_len);
 
 #ifdef __cplusplus
 }

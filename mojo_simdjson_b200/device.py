@@ -20,6 +20,42 @@ class DeviceResult:
     utf8_error: int
 
 
+def pointer_program(pointers) -> tuple[bytes, "C.Array"]:
+    """The pointers (str or bytes) as the flat byte string and the K + 1 offsets the C entry points take."""
+    raw = [p.encode("utf-8") if isinstance(p, str) else bytes(p) for p in pointers]
+    offs = [0]
+    for p in raw:
+        offs.append(offs[-1] + len(p))
+    return b"".join(raw), (C.c_uint64 * len(offs))(*offs)
+
+
+@dataclass
+class PointerColumns:
+    """K columns of D cells from Stage1Context.at_pointers, each a [K, D] device tensor (include/simdjson_b200.h,
+    sjb200_at_pointers_device_async): type (uint8, the tape type character or 0), code (uint8, 0 = found), value (int64)."""
+    type: torch.Tensor
+    code: torch.Tensor
+    value: torch.Tensor
+
+    def int64(self, k: int) -> tuple[torch.Tensor, torch.Tensor]:
+        """(values, mask) of column k: the integers of 'l' cells, 0 elsewhere."""
+        mask = self.type[k] == ord("l")
+        return torch.where(mask, self.value[k], torch.zeros_like(self.value[k])), mask
+
+    def float64(self, k: int) -> tuple[torch.Tensor, torch.Tensor]:
+        """(values, mask) of column k: 'd' cells bit-cast, 'l' cells converted as float(int) would (nearest), 0 elsewhere."""
+        t, v = self.type[k], self.value[k]
+        is_d, is_l = t == ord("d"), t == ord("l")
+        out = torch.where(is_d, v.view(torch.float64), v.to(torch.float64))
+        mask = is_d | is_l
+        return torch.where(mask, out, torch.zeros_like(out)), mask
+
+    def boolean(self, k: int) -> tuple[torch.Tensor, torch.Tensor]:
+        """(values, mask) of column k: True for 't' cells, False for 'f' cells and everywhere else."""
+        t = self.type[k]
+        return t == ord("t"), (t == ord("t")) | (t == ord("f"))
+
+
 class Stage1Context:
     """One parser context per GPU; runs on torch's current stream of that device by default."""
 
@@ -186,6 +222,42 @@ class Stage1Context:
             raise RuntimeError(f"stage-2 stream walk failed: {errors.NAMES.get(rc, rc)}")
         nd = int(summary[0].item())
         return {"tape": tape, "doc_first": first[: nd + 1], "doc_tape": doc_tape[: nd + 1], "doc_status": status[:nd], "summary": summary}
+
+    def at_pointers(self, pointers, tape: torch.Tensor, string_buf: torch.Tensor, doc_tape: torch.Tensor, doc_status: torch.Tensor) -> PointerColumns:
+        """JSON Pointer lookups (RFC 6901) on device tapes, one column per pointer over every document (include/simdjson_b200.h,
+        sjb200_at_pointers_device_async, for the rules).  `pointers`: str or bytes.  Enqueued on the context's stream; the
+        tape stays on the device.  Over a stream of documents:
+
+            prims = ctx.stage2_primitives(buf, idx, n)
+            s = ctx.stage2_stream(buf, idx, n, prims)
+            cols = ctx.at_pointers(["/user/id", "/text"], s["tape"], prims["string_buf"], s["doc_tape"], s["doc_status"])
+            ids, found = cols.int64(0)
+
+        Over one document (D = 1):
+
+            tape, summary = ctx.stage2_tape(buf, idx, n, prims)
+            doc_tape = torch.stack([torch.zeros_like(summary[2]), summary[2]])
+            cols = ctx.at_pointers(["/a/0"], tape, prims["string_buf"], doc_tape, summary[:1])
+
+        The whole `tape` and `string_buf` tensors bound the reads.  Raises ValueError for an invalid pointer or one over the
+        limits (SJB200_POINTER_MAX_COUNT, SJB200_POINTER_MAX_BYTES)."""
+        for t, dt in ((tape, torch.int64), (doc_tape, torch.int64), (doc_status, torch.int64), (string_buf, torch.uint8)):
+            assert t.is_cuda and t.dtype == dt and t.is_contiguous()
+        n_docs = doc_status.numel()
+        assert doc_tape.numel() >= n_docs + 1
+        raw, offs = pointer_program(pointers)
+        k = len(offs) - 1
+        dev = tape.device
+        cols = PointerColumns(torch.zeros((k, n_docs), dtype=torch.uint8, device=dev), torch.zeros((k, n_docs), dtype=torch.uint8, device=dev),
+                              torch.zeros((k, n_docs), dtype=torch.int64, device=dev))
+        rc = self._lib.sjb200_at_pointers_device_async(self._ctx, tape.data_ptr(), tape.numel(), string_buf.data_ptr(), string_buf.numel(),
+                                                       doc_tape.data_ptr(), doc_status.data_ptr(), n_docs, raw, offs, k, cols.type.data_ptr(),
+                                                       cols.code.data_ptr(), cols.value.data_ptr())
+        if rc in (errors.INVALID_JSON_POINTER, errors.CAPACITY):
+            raise ValueError(f"pointer lookup refused: {errors.NAMES[rc]}")
+        if rc != errors.SUCCESS:
+            raise RuntimeError(f"pointer lookup failed: {errors.NAMES.get(rc, rc)}")
+        return cols
 
     def last_elapsed_ms(self) -> float:
         return float(self._lib.sjb200_last_elapsed_ms(self._ctx))

@@ -94,6 +94,29 @@ class DocumentStream:
         return doc
 
 
+class PointerCells:
+    """The result of DomParserImplementation.at_pointers(): K columns of D cells as numpy arrays [K, D] (include/simdjson_b200.h,
+    sjb200_stage2_stream_at_pointers), and the stream's string buffer that string cells point into."""
+
+    def __init__(self, type_, code, value, string_buf):
+        self.type = type_           # uint8: the tape type character of the value found, 0 if not found
+        self.code = code            # uint8: 0 = found, else the simdjson error code
+        self.value = value          # int64: integer, double bits, 1/0 for true/false/null, string record offset, container index
+        self.string_buf = string_buf
+
+    def strings(self, k: int) -> list:
+        """Column k as bytes for string cells, None for every other cell."""
+        sb = self.string_buf
+        out = []
+        for t, off in zip(self.type[k].tolist(), self.value[k].tolist()):
+            if t == ord('"'):
+                n = int.from_bytes(sb[off : off + 4].tobytes(), "little")
+                out.append(sb[off + 4 : off + 4 + n].tobytes())
+            else:
+                out.append(None)
+        return out
+
+
 class DomParserImplementation:
     """Stage-1 half of the reference's DomParserImplementation, backed by the B200 kernel."""
 
@@ -108,6 +131,7 @@ class DomParserImplementation:
         self.next_structural_index = 0
         self.document = Document()
         self.stream: DocumentStream | None = None    # stage2_stream()'s result
+        self.pointer_cells: PointerCells | None = None   # at_pointers()'s result
         self.utf8_error = 0                          # not in the reference: its Utf8Checker is a stub
         self._capacity = 0
         self._max_depth = 100
@@ -203,4 +227,33 @@ class DomParserImplementation:
         if rc == errors.SUCCESS:
             d = int(nd.value)
             self.stream = DocumentStream(tape[: tl.value], sbuf[: sl.value], first[: d + 1], doc_tape[: d + 1], status[:d], int(nf.value), int(inexact.value))
+        return rc
+
+    def at_pointers(self, pointers) -> int:
+        """JSON Pointer lookups over every document of the stream stage1() indexed (include/simdjson_b200.h for the rules): the
+        walk and the lookups run on the device and only the cells and the string buffer come back, into `self.pointer_cells`
+        (a PointerCells).  `pointers`: str or bytes.  Returns the call's code: SUCCESS also when cells hold errors;
+        INVALID_JSON_POINTER or CAPACITY for pointers the call refuses."""
+        from .device import pointer_program
+
+        n, length = int(self.n_structural_indexes), int(self.length)
+        if self.buf is None or n == 0:
+            return errors.UNINITIALIZED
+        raw, offs = pointer_program(pointers)
+        k = len(offs) - 1
+        docs = int(np.count_nonzero(self.buf == 0x0A)) + 1    # a first guess; the call reports the real count
+        sb_cap = length + 2 * n + 64
+        nd, sl = C.c_uint64(0), C.c_uint64(0)
+        for _ in range(2):
+            cells = max(k * docs, 1)
+            ty, code, val = np.zeros(cells, np.uint8), np.zeros(cells, np.uint8), np.zeros(cells, np.int64)
+            sbuf = np.zeros(sb_cap, dtype=np.uint8)
+            rc = self._lib.sjb200_stage2_stream_at_pointers(self._ctx, raw, offs, k, ty.ctypes.data, code.ctypes.data, val.ctypes.data, cells,
+                                                            sbuf.ctypes.data, sbuf.size, C.byref(nd), C.byref(sl))
+            if rc != errors.CAPACITY or k * int(nd.value) <= cells and int(sl.value) <= sb_cap:
+                break
+            docs, sb_cap = int(nd.value), int(sl.value)
+        if rc == errors.SUCCESS:
+            d = int(nd.value)
+            self.pointer_cells = PointerCells(ty[: k * d].reshape(k, d), code[: k * d].reshape(k, d), val[: k * d].reshape(k, d), sbuf[: sl.value])
         return rc
