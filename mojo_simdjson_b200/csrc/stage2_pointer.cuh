@@ -229,6 +229,29 @@ __global__ void __launch_bounds__(PTR_THREADS) at_pointer_kernel(const uint64_t 
     out_value[cell] = value;
 }
 
+// sjb200_at_pointers_device_async after the compilation of its pointers
+int32_t at_pointers_enqueue(sjb200_ctx *c, const PtrProgram &prog, uint64_t n_pointers, const uint64_t *d_tape, uint64_t tape_len, const uint8_t *d_strbuf,
+                            uint64_t strbuf_len, const uint64_t *d_doc_tape, const uint64_t *d_doc_status, uint64_t n_docs, uint8_t *d_type, uint8_t *d_code,
+                            int64_t *d_value) {
+    if (n_docs == 0 || n_pointers == 0) return SJB200_SUCCESS;
+    if (!d_tape || !d_strbuf || !d_doc_tape || !d_doc_status || !d_type || !d_code || !d_value) return SJB200_UNINITIALIZED;
+    if (n_docs >= (1ull << 40)) return SJB200_CAPACITY;
+    CK(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    const size_t bytes = prog.words.size() * 4;
+    PoolBuffers tmp(c);
+    uint32_t *d_prog = tmp.get<uint32_t>(prog.words.size());
+    if (tmp.failed) return SJB200_MEMALLOC;
+    // pageable source: the copy has taken the bytes when it returns, so `prog` may go out of scope
+    CK(cudaMemcpyAsync(d_prog, prog.words.data(), bytes, cudaMemcpyHostToDevice, s));
+    if (prog.smem > 48 * 1024) CK(cudaFuncSetAttribute(at_pointer_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prog.smem));
+    const dim3 grid((unsigned)((n_docs + PTR_THREADS - 1) / PTR_THREADS), (unsigned)n_pointers);
+    at_pointer_kernel<<<grid, PTR_THREADS, prog.smem, s>>>(d_tape, tape_len, d_strbuf, strbuf_len, d_doc_tape, d_doc_status, n_docs, d_prog, (uint32_t)n_pointers,
+                                                          d_type, d_code, d_value);
+    c->launches += 1;
+    return cuda_err(cudaGetLastError());
+}
+
 }  // namespace
 
 #pragma GCC visibility push(default)
@@ -239,32 +262,9 @@ int32_t sjb200_at_pointers_device_async(sjb200_ctx *c, const uint64_t *d_tape, u
                                         const uint64_t *pointer_offsets, uint64_t n_pointers, uint8_t *d_type, uint8_t *d_code, int64_t *d_value) {
     if (!c || !pointer_offsets || (!pointers && n_pointers)) return SJB200_UNINITIALIZED;
     PtrProgram prog;
-    int32_t rc = ptr_compile(pointers, pointer_offsets, n_pointers, prog);
+    const int32_t rc = ptr_compile(pointers, pointer_offsets, n_pointers, prog);
     if (rc != SJB200_SUCCESS) return rc;
-    if (n_docs == 0 || n_pointers == 0) return SJB200_SUCCESS;
-    if (!d_tape || !d_strbuf || !d_doc_tape || !d_doc_status || !d_type || !d_code || !d_value) return SJB200_UNINITIALIZED;
-    if (n_docs >= (1ull << 40)) return SJB200_CAPACITY;
-    CK(cudaSetDevice(c->device));
-    cudaStream_t s = c->stream;
-    uint32_t *d_prog = nullptr;
-    const size_t bytes = prog.words.size() * 4;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_prog, bytes, c->pool, s);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return SJB200_MEMALLOC;
-    }
-    // pageable source: the copy has taken the bytes when it returns, so `prog` may go out of scope
-    e = cudaMemcpyAsync(d_prog, prog.words.data(), bytes, cudaMemcpyHostToDevice, s);
-    if (e == cudaSuccess && prog.smem > 48 * 1024) e = cudaFuncSetAttribute(at_pointer_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prog.smem);
-    if (e == cudaSuccess) {
-        const dim3 grid((unsigned)((n_docs + PTR_THREADS - 1) / PTR_THREADS), (unsigned)n_pointers);
-        at_pointer_kernel<<<grid, PTR_THREADS, prog.smem, s>>>(d_tape, tape_len, d_strbuf, strbuf_len, d_doc_tape, d_doc_status, n_docs, d_prog,
-                                                              (uint32_t)n_pointers, d_type, d_code, d_value);
-        e = cudaGetLastError();
-        c->launches += 1;
-    }
-    cudaFreeAsync(d_prog, s);
-    return e == cudaSuccess ? SJB200_SUCCESS : cuda_err(e);
+    return at_pointers_enqueue(c, prog, n_pointers, d_tape, tape_len, d_strbuf, strbuf_len, d_doc_tape, d_doc_status, n_docs, d_type, d_code, d_value);
 }
 
 // Host to host: the stream walk of the document the preceding sjb200_stage1 left resident, then the lookups; only the cells
@@ -274,87 +274,33 @@ int32_t sjb200_stage2_stream_at_pointers(sjb200_ctx *c, const uint8_t *pointers,
                                          uint64_t *n_docs, uint64_t *strbuf_len) {
     if (!c || !pointer_offsets || (!pointers && n_pointers)) return SJB200_UNINITIALIZED;
     if (n_pointers && (!type_out || !code_out || !value_out)) return SJB200_UNINITIALIZED;
-    if (c->resident_len == 0 || c->resident_n == 0) return SJB200_UNINITIALIZED;   // no successful stage 1 before this call
-    {
-        PtrProgram check;   // refuse a bad pointer before any work
-        const int32_t rc = ptr_compile(pointers, pointer_offsets, n_pointers, check);
-        if (rc != SJB200_SUCCESS) return rc;
-    }
-    const uint64_t len = c->resident_len, n = c->resident_n;
-    CK(cudaSetDevice(c->device));
+    PtrProgram prog;   // compiled once, and first: a bad pointer is refused before any device work
+    int32_t rc = ptr_compile(pointers, pointer_offsets, n_pointers, prog);
+    if (rc != SJB200_SUCCESS) return rc;
+    PoolBuffers tmp(c);
+    ResidentStage2 r;
+    rc = stage2_resident<true>(c, tmp, r);
+    if (rc != SJB200_SUCCESS) return rc;
+    const uint64_t nd = r.sum.n_docs, sb = r.sum.strbuf_len, cells = n_pointers * nd;
+    if (n_docs) *n_docs = nd;
+    if (strbuf_len) *strbuf_len = sb;
+    if (cells > cells_capacity || (strbuf_out && sb > strbuf_capacity)) return SJB200_CAPACITY;
     cudaStream_t s = c->stream;
-    const uint64_t sb_cap = len + 2 * n + 64, tp_cap = 4 * n;
-    uint8_t *d_kind = nullptr, *d_err = nullptr, *d_sb = nullptr, *d_cells = nullptr;
-    int64_t *d_val = nullptr;
-    uint64_t *d_off = nullptr, *d_tape = nullptr, *d_sum = nullptr, *d_dtape = nullptr, *d_dstatus = nullptr;
-    uint32_t *d_dfirst = nullptr;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_kind, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_err, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_val, n * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_off, n * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sb, sb_cap, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tape, tp_cap * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sum, 64, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dfirst, (n + 1) * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dtape, (n + 1) * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dstatus, n * 8, c->pool, s);
-    auto release = [&]() {
-        if (d_kind) cudaFreeAsync(d_kind, s);
-        if (d_err) cudaFreeAsync(d_err, s);
-        if (d_val) cudaFreeAsync(d_val, s);
-        if (d_off) cudaFreeAsync(d_off, s);
-        if (d_sb) cudaFreeAsync(d_sb, s);
-        if (d_tape) cudaFreeAsync(d_tape, s);
-        if (d_sum) cudaFreeAsync(d_sum, s);
-        if (d_dfirst) cudaFreeAsync(d_dfirst, s);
-        if (d_dtape) cudaFreeAsync(d_dtape, s);
-        if (d_dstatus) cudaFreeAsync(d_dstatus, s);
-        if (d_cells) cudaFreeAsync(d_cells, s);
-    };
-    if (e != cudaSuccess) {
-        release();
-        cudaGetLastError();
-        return SJB200_MEMALLOC;
+    if (cells) {
+        // [K][D] codes, then types, then values (8-byte aligned at 2 cells bytes rounded up)
+        const uint64_t voff = (2 * cells + 7) & ~7ull;
+        uint8_t *d_cells = tmp.get<uint8_t>(voff + 8 * cells);
+        if (tmp.failed) return SJB200_MEMALLOC;
+        rc = at_pointers_enqueue(c, prog, n_pointers, r.tape, r.sum.tape_len, r.strbuf, sb, r.doc_tape, r.doc_status, nd, d_cells + cells, d_cells,
+                                 reinterpret_cast<int64_t *>(d_cells + voff));
+        if (rc != SJB200_SUCCESS) return rc;
+        CK(cudaMemcpyAsync(code_out, d_cells, cells, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(type_out, d_cells + cells, cells, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(value_out, d_cells + voff, 8 * cells, cudaMemcpyDeviceToHost, s));
     }
-    int32_t rc = sjb200_stage2_primitives_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_sb, sb_cap, d_sum);
-    if (rc == SJB200_SUCCESS)
-        rc = sjb200_stage2_stream_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_tape, tp_cap, d_dfirst, d_dtape, d_dstatus, d_sum + 4);
-    uint64_t sum[8] = {};
-    if (rc == SJB200_SUCCESS) {
-        e = cudaMemcpyAsync(sum, d_sum, 64, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) rc = cuda_err(e);
-    }
-    if (rc == SJB200_SUCCESS) {
-        const uint64_t sb = sum[1], nd = sum[4], tl = sum[6], cells = n_pointers * nd;
-        if (n_docs) *n_docs = nd;
-        if (strbuf_len) *strbuf_len = sb;
-        if (cells > cells_capacity || (strbuf_out && sb > strbuf_capacity)) rc = SJB200_CAPACITY;
-        if (rc == SJB200_SUCCESS && cells) {
-            // [K][D] codes, then types, then values (8-byte aligned at 2 cells bytes rounded up)
-            const uint64_t voff = (2 * cells + 7) & ~7ull;
-            e = cudaMallocFromPoolAsync(&d_cells, voff + 8 * cells, c->pool, s);
-            if (e != cudaSuccess) {
-                cudaGetLastError();
-                rc = SJB200_MEMALLOC;
-            } else {
-                rc = sjb200_at_pointers_device_async(c, d_tape, tl, d_sb, sb, d_dtape, d_dstatus, nd, pointers, pointer_offsets, n_pointers, d_cells + cells,
-                                                     d_cells, reinterpret_cast<int64_t *>(d_cells + voff));
-                if (rc == SJB200_SUCCESS) {
-                    e = cudaMemcpyAsync(code_out, d_cells, cells, cudaMemcpyDeviceToHost, s);
-                    if (e == cudaSuccess) e = cudaMemcpyAsync(type_out, d_cells + cells, cells, cudaMemcpyDeviceToHost, s);
-                    if (e == cudaSuccess) e = cudaMemcpyAsync(value_out, d_cells + voff, 8 * cells, cudaMemcpyDeviceToHost, s);
-                }
-            }
-        }
-        if (rc == SJB200_SUCCESS && strbuf_out && sb) e = cudaMemcpyAsync(strbuf_out, d_sb, sb, cudaMemcpyDeviceToHost, s);
-        if (rc == SJB200_SUCCESS) {
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e != cudaSuccess) rc = cuda_err(e);
-        }
-    }
-    release();
-    return rc;
+    if (strbuf_out && sb) CK(cudaMemcpyAsync(strbuf_out, r.strbuf, sb, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return SJB200_SUCCESS;
 }
 
 }  // extern "C"

@@ -22,6 +22,8 @@
 // First slice: one thread walks one string byte by byte; a document that is one enormous string is correct but slow.
 #pragma once
 
+#include <vector>
+
 namespace {
 
 enum : uint8_t { S2_NONE = 0, S2_STRING = 1, S2_INT = 2, S2_FLOAT = 3, S2_TRUE = 4, S2_FALSE = 5, S2_NULL = 6, S2_BAD = 7 };
@@ -226,19 +228,20 @@ __global__ void __launch_bounds__(256) stage2_primitives_kernel(const uint8_t *_
     }
 }
 
-// ---- exclusive prefix sum of uint64 (in place), three launches: per-block totals, one CTA over the totals, per-block scan ----
+// ---- exclusive prefix sum (in place), three launches: per-block totals, one CTA over the totals, per-block scan ----
 constexpr int SCAN_THREADS = 256, SCAN_PER_THREAD = 8, SCAN_BLOCK = SCAN_THREADS * SCAN_PER_THREAD;
 
-__device__ __forceinline__ uint64_t scan_block_exclusive(uint64_t mine, uint64_t *s_w, uint64_t &total) {   // over the CTA's 256 threads
-    uint64_t incl = mine;
+template <typename T>
+__device__ __forceinline__ T scan_block_exclusive(T mine, T *s_w, T &total) {   // over the CTA's 256 threads
+    T incl = mine;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
-        const uint64_t o = __shfl_up_sync(0xFFFFFFFFu, incl, d);
+        const T o = __shfl_up_sync(0xFFFFFFFFu, incl, d);
         if ((int)(threadIdx.x & 31) >= d) incl += o;
     }
     if ((threadIdx.x & 31) == 31) s_w[threadIdx.x >> 5] = incl;
     __syncthreads();
-    uint64_t before = 0, all = 0;
+    T before = 0, all = 0;
     for (int q = 0; q < SCAN_THREADS / 32; q++) {
         if (q < (int)(threadIdx.x >> 5)) before += s_w[q];
         all += s_w[q];
@@ -247,14 +250,15 @@ __device__ __forceinline__ uint64_t scan_block_exclusive(uint64_t mine, uint64_t
     __syncthreads();
     return before + incl - mine;
 }
-__global__ void __launch_bounds__(SCAN_THREADS) scan_totals_kernel(const uint64_t *__restrict__ x, uint64_t n, uint64_t *__restrict__ block_total) {
-    __shared__ uint64_t s_w[SCAN_THREADS / 32];
+template <typename T>
+__global__ void __launch_bounds__(SCAN_THREADS) scan_totals_kernel(const T *__restrict__ x, uint64_t n, uint64_t *__restrict__ block_total) {
+    __shared__ T s_w[SCAN_THREADS / 32];
     const uint64_t k0 = (uint64_t)blockIdx.x * SCAN_BLOCK + (uint64_t)threadIdx.x * SCAN_PER_THREAD;
-    uint64_t mine = 0;
+    T mine = 0;
 #pragma unroll
     for (int j = 0; j < SCAN_PER_THREAD; j++)
         if (k0 + j < n) mine += x[k0 + j];
-    uint64_t total;
+    T total;
     scan_block_exclusive(mine, s_w, total);
     if (threadIdx.x == 0) block_total[blockIdx.x] = total;
 }
@@ -284,22 +288,71 @@ __global__ void __launch_bounds__(1024) scan_of_totals_kernel(uint64_t *block_to
     }
     if (threadIdx.x == 0) *grand_total = s_carry;
 }
-__global__ void __launch_bounds__(SCAN_THREADS) scan_apply_kernel(uint64_t *__restrict__ x, uint64_t n, const uint64_t *__restrict__ block_before) {
-    __shared__ uint64_t s_w[SCAN_THREADS / 32];
+template <typename T>
+__global__ void __launch_bounds__(SCAN_THREADS) scan_apply_kernel(T *__restrict__ x, uint64_t n, const uint64_t *__restrict__ block_before) {
+    __shared__ T s_w[SCAN_THREADS / 32];
     const uint64_t k0 = (uint64_t)blockIdx.x * SCAN_BLOCK + (uint64_t)threadIdx.x * SCAN_PER_THREAD;
-    uint64_t v[SCAN_PER_THREAD], mine = 0;
+    T v[SCAN_PER_THREAD], mine = 0;
 #pragma unroll
     for (int j = 0; j < SCAN_PER_THREAD; j++) {
         v[j] = k0 + j < n ? x[k0 + j] : 0;
         mine += v[j];
     }
-    uint64_t total;
-    uint64_t run = block_before[blockIdx.x] + scan_block_exclusive(mine, s_w, total);
+    T total;
+    T run = (T)block_before[blockIdx.x] + scan_block_exclusive(mine, s_w, total);
 #pragma unroll
     for (int j = 0; j < SCAN_PER_THREAD; j++) {
         if (k0 + j < n) x[k0 + j] = run;
         run += v[j];
     }
+}
+
+// The temporaries of one call, from the context's stream-ordered pool.  Hands out buffers until an allocation fails (from
+// then on nullptr, with `failed` set and the CUDA error cleared); frees everything it handed out, stream ordered, when it
+// goes out of scope.
+struct PoolBuffers {
+    explicit PoolBuffers(sjb200_ctx *c) : pool(c->pool), s(c->stream) {}
+    PoolBuffers(const PoolBuffers &) = delete;
+    PoolBuffers &operator=(const PoolBuffers &) = delete;
+    ~PoolBuffers() {
+        for (void *p : bufs) cudaFreeAsync(p, s);
+    }
+    template <typename T>
+    T *get(uint64_t count) {
+        void *p = nullptr;
+        if (failed) return nullptr;
+        if (cudaMallocFromPoolAsync(&p, count * sizeof(T), pool, s) != cudaSuccess) {
+            failed = true;
+            cudaGetLastError();
+            return nullptr;
+        }
+        bufs.push_back(p);
+        return static_cast<T *>(p);
+    }
+    cudaMemPool_t pool;
+    cudaStream_t s;
+    std::vector<void *> bufs;
+    bool failed = false;
+};
+
+// exclusive scan of x[0 .. n) in place on the context's stream; *d_total (device) receives the grand total
+template <typename T>
+int32_t scan_exclusive(T *x, uint64_t n, unsigned long long *d_total, sjb200_ctx *c) {
+    const uint64_t nblocks = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    PoolBuffers tmp(c);
+    uint64_t *d_totals = tmp.get<uint64_t>(nblocks);
+    if (tmp.failed) return SJB200_MEMALLOC;
+    scan_totals_kernel<<<(unsigned)nblocks, SCAN_THREADS, 0, c->stream>>>(x, n, d_totals);
+    scan_of_totals_kernel<<<1, 1024, 0, c->stream>>>(d_totals, (uint32_t)nblocks, d_total);
+    scan_apply_kernel<<<(unsigned)nblocks, SCAN_THREADS, 0, c->stream>>>(x, n, d_totals);
+    c->launches += 3;
+    return cuda_err(cudaGetLastError());
+}
+
+// the grid of a grid-stride kernel of 256 threads over n items: one thread per item, at most 32 CTAs per SM
+unsigned grid_256(const sjb200_ctx *c, uint64_t n) {
+    const uint64_t blocks = (n + 255) / 256, cap = (uint64_t)c->sm_count * 32;
+    return (unsigned)(blocks < cap ? blocks : cap);
 }
 
 // every string's record {uint32 length, bytes} at strbuf + off[k]; a string that failed gets length 0
@@ -337,19 +390,12 @@ int32_t sjb200_stage2_primitives_device_async(sjb200_ctx *c, const uint8_t *d_bu
     CK(cudaMemsetAsync(d_summary, 0xFF, 8, s));
     CK(cudaMemsetAsync(d_summary + 1, 0, 24, s));
     if (n == 0) return SJB200_SUCCESS;
-    const unsigned grid = (unsigned)((n + 255) / 256 < (uint64_t)c->sm_count * 32 ? (n + 255) / 256 : (uint64_t)c->sm_count * 32);
+    const unsigned grid = grid_256(c, n);
     stage2_primitives_kernel<<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_value, d_str_off, reinterpret_cast<unsigned long long *>(d_summary));
     CK(cudaGetLastError());
-    const uint64_t nblocks = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
-    uint64_t *d_totals = nullptr;
-    CK(cudaMallocFromPoolAsync(&d_totals, nblocks * 8, c->pool, s));
-    scan_totals_kernel<<<(unsigned)nblocks, SCAN_THREADS, 0, s>>>(d_str_off, n, d_totals);
-    scan_of_totals_kernel<<<1, 1024, 0, s>>>(d_totals, (uint32_t)nblocks, reinterpret_cast<unsigned long long *>(d_summary + 1));
-    scan_apply_kernel<<<(unsigned)nblocks, SCAN_THREADS, 0, s>>>(d_str_off, n, d_totals);
-    cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(d_totals, s);
-    if (e != cudaSuccess) return cuda_err(e);
-    c->launches += 4;
+    c->launches += 1;
+    const int32_t rc = scan_exclusive(d_str_off, n, reinterpret_cast<unsigned long long *>(d_summary + 1), c);
+    if (rc != SJB200_SUCCESS) return rc;
     if (d_strbuf) {
         stage2_strings_kernel<<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_value, d_str_off, d_strbuf, strbuf_capacity);
         CK(cudaGetLastError());

@@ -558,65 +558,125 @@ __global__ void __launch_bounds__(256) stream_failed_kernel(const unsigned long 
     }
 }
 
-// ---- exclusive prefix sum of uint32 (in place), same three launches as the uint64 one of stage2_primitives.cuh ----
-__device__ __forceinline__ uint32_t scan32_block_exclusive(uint32_t mine, uint32_t *s_w, uint32_t &total) {
-    uint32_t incl = mine;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t o = __shfl_up_sync(0xFFFFFFFFu, incl, d);
-        if ((int)(threadIdx.x & 31) >= d) incl += o;
+// The walk over a single document (STREAM false) or a stream of documents: the buffers and the launch sequence of both
+// modes, with the steps only a stream needs behind `if constexpr`.  The caller has checked the arguments and initialised
+// the summary (and, STREAM, the document status words).
+template <bool STREAM>
+int32_t stage2_walk(sjb200_ctx *c, const uint8_t *d_buf, uint64_t len, const uint32_t *d_idx, uint64_t n, const uint8_t *d_kind, const uint8_t *d_err,
+                    const int64_t *d_value, const uint64_t *d_str_off, uint64_t *d_tape, uint64_t tape_capacity, unsigned long long *summary,
+                    uint32_t *d_doc_first, uint64_t *d_doc_tape, unsigned long long *doc_status) {
+    cudaStream_t s = c->stream;
+    const uint64_t nblk = (n + TAPE_BLOCK - 1) / TAPE_BLOCK, dblk = (n + DEPTH_BLOCK - 1) / DEPTH_BLOCK;
+    const uint32_t ntiles = (uint32_t)((n + MS_TILE - 1) / MS_TILE);
+    const uint64_t hist_half = (uint64_t)MS_CLASSES * ntiles;   // hist: the B part, then the A part
+    PoolBuffers tmp(c);
+    Stk *d_stk = tmp.get<Stk>(nblk);
+    uint32_t *d_words = tmp.get<uint32_t>(n);
+    uint8_t *d_cls = tmp.get<uint8_t>(n);
+    uint32_t *d_slot = tmp.get<uint32_t>(n), *d_rank = tmp.get<uint32_t>(n), *d_sorted = tmp.get<uint32_t>(n), *d_hist = tmp.get<uint32_t>(2 * hist_half);
+    unsigned long long *d_tot = tmp.get<unsigned long long>(4);
+    uint32_t *d_doc = STREAM ? tmp.get<uint32_t>(n) : nullptr;
+    uint8_t *d_bytes = STREAM ? tmp.get<uint8_t>(n) : nullptr, *d_starts = STREAM ? tmp.get<uint8_t>(n) : nullptr;
+    int32_t *d_depth = STREAM ? tmp.get<int32_t>(dblk) : nullptr;
+    if (tmp.failed) return SJB200_MEMALLOC;
+    const unsigned grid = grid_256(c, n);
+    StreamArgs sa{};
+    int32_t rc;
+    if constexpr (STREAM) {
+        // where documents start: the bracket depth over the structural bytes
+        rc = sjb200_structural_bytes_device_async(c, d_buf, len, d_idx, n, d_bytes);
+        if (rc == SJB200_SUCCESS) rc = sjb200_document_starts_device_async(c, d_bytes, n, d_starts, d_depth, dblk);
+        if (rc != SJB200_SUCCESS) return rc;
+        // the document of every token, and the first token of every document
+        stream_flags_kernel<<<grid, 256, 0, s>>>(d_starts, n, d_doc);
+        c->launches += 1;
+        rc = scan_exclusive(d_doc, n, summary, c);
+        if (rc != SJB200_SUCCESS) return rc;
+        stream_docs_kernel<<<grid, 256, 0, s>>>(d_starts, n, d_doc, d_doc_first, summary);
+        c->launches += 1;
+        sa = StreamArgs{d_starts, d_doc, d_doc_first, d_doc_tape, doc_status};
     }
-    if ((threadIdx.x & 31) == 31) s_w[threadIdx.x >> 5] = incl;
-    __syncthreads();
-    uint32_t before = 0, all = 0;
-    for (int q = 0; q < SCAN_THREADS / 32; q++) {
-        if (q < (int)(threadIdx.x >> 5)) before += s_w[q];
-        all += s_w[q];
+    // depth / container type (inside each document): the bit-stack scan; then the grammar, the words and the multisplit classes
+    tape_stack_totals_kernel<STREAM><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_stk, sa.starts);
+    tape_stack_scan_kernel<STREAM><<<1, 1024, 0, s>>>(d_stk, (uint32_t)nblk);
+    tape_grammar_kernel<STREAM><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_stk, d_words, d_cls, STREAM ? nullptr : summary, sa);
+    c->launches += 3;
+    // where every token's words go; their total is summary[1] of the single walk (the stream's [1] counts failing documents)
+    rc = scan_exclusive(d_words, n, STREAM ? d_tot + 2 : summary + 1, c);
+    if (rc != SJB200_SUCCESS) return rc;
+    if constexpr (STREAM) {
+        stream_roots_kernel<<<grid, 256, 0, s>>>(d_doc_first, d_words, n, summary, d_tot + 2, d_doc_tape, d_tape, tape_capacity, summary);
+        c->launches += 1;
     }
-    total = all;
-    __syncthreads();
-    return before + incl - mine;
+    // brackets and commas by depth: two class-major histograms, each scanned on its own, then the ranks
+    tape_multisplit_hist_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist);
+    c->launches += 1;
+    rc = scan_exclusive(d_hist, hist_half, d_tot, c);                                            // B: total = number of brackets
+    if (rc == SJB200_SUCCESS) rc = scan_exclusive(d_hist + hist_half, hist_half, d_tot + 1, c);   // A
+    if (rc != SJB200_SUCCESS) return rc;
+    tape_multisplit_rank_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist, 0u, d_slot, d_rank, d_sorted);
+    tape_emit_kernel<STREAM><<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_value, d_str_off, d_words, d_cls, d_slot, d_rank, d_sorted, (uint32_t)n,
+                                                  d_tape, tape_capacity, summary, sa);
+    if constexpr (STREAM) stream_failed_kernel<<<grid, 256, 0, s>>>(doc_status, summary);
+    else tape_roots_kernel<<<1, 1, 0, s>>>(d_tape, tape_capacity, summary + 1, summary);
+    c->launches += 3;
+    return cuda_err(cudaGetLastError());
 }
-__global__ void __launch_bounds__(SCAN_THREADS) scan32_totals_kernel(const uint32_t *__restrict__ x, uint64_t n, uint64_t *__restrict__ block_total) {
-    __shared__ uint32_t s_w[SCAN_THREADS / 32];
-    const uint64_t k0 = (uint64_t)blockIdx.x * SCAN_BLOCK + (uint64_t)threadIdx.x * SCAN_PER_THREAD;
-    uint32_t mine = 0;
-#pragma unroll
-    for (int j = 0; j < SCAN_PER_THREAD; j++)
-        if (k0 + j < n) mine += x[k0 + j];
-    uint32_t total;
-    scan32_block_exclusive(mine, s_w, total);
-    if (threadIdx.x == 0) block_total[blockIdx.x] = total;
-}
-__global__ void __launch_bounds__(SCAN_THREADS) scan32_apply_kernel(uint32_t *__restrict__ x, uint64_t n, const uint64_t *__restrict__ block_before) {
-    __shared__ uint32_t s_w[SCAN_THREADS / 32];
-    const uint64_t k0 = (uint64_t)blockIdx.x * SCAN_BLOCK + (uint64_t)threadIdx.x * SCAN_PER_THREAD;
-    uint32_t v[SCAN_PER_THREAD], mine = 0;
-#pragma unroll
-    for (int j = 0; j < SCAN_PER_THREAD; j++) {
-        v[j] = k0 + j < n ? x[k0 + j] : 0;
-        mine += v[j];
+
+// What a host-to-host call reads back: the summary of sjb200_stage2_primitives_device_async, then the walk's
+struct Stage2Summary {
+    uint64_t first_primitive_error, strbuf_len, primitives_unused[2];
+    union {
+        uint64_t verdict;   // single walk: first error, all ones = SUCCESS
+        uint64_t n_docs;    // stream walk
+    };
+    union {
+        uint64_t token_words;
+        uint64_t n_failed;
+    };
+    uint64_t tape_len, inexact_doubles;
+};
+static_assert(sizeof(Stage2Summary) == 64, "two summaries of 4 words");
+
+// The device results of a host-to-host call, in buffers of the caller's PoolBuffers
+struct ResidentStage2 {
+    uint8_t *strbuf = nullptr;
+    uint64_t *tape = nullptr, *doc_tape = nullptr, *doc_status = nullptr;
+    uint32_t *doc_first = nullptr;
+    Stage2Summary sum = {};
+};
+
+// The part the host-to-host calls share: primitives and the walk over the document the preceding successful sjb200_stage1 on
+// this context left on the device (no second copy of the input), then both summaries read back.  Synchronous.
+template <bool STREAM>
+int32_t stage2_resident(sjb200_ctx *c, PoolBuffers &tmp, ResidentStage2 &r) {
+    if (c->resident_len == 0 || c->resident_n == 0) return SJB200_UNINITIALIZED;   // no successful stage 1 before this call
+    const uint64_t len = c->resident_len, n = c->resident_n;
+    CK(cudaSetDevice(c->device));
+    const uint64_t sb_cap = len + 2 * n + 64, tp_cap = STREAM ? 4 * n : 2 * n + 2;
+    uint8_t *d_kind = tmp.get<uint8_t>(n), *d_err = tmp.get<uint8_t>(n);
+    int64_t *d_val = tmp.get<int64_t>(n);
+    uint64_t *d_off = tmp.get<uint64_t>(n);
+    r.strbuf = tmp.get<uint8_t>(sb_cap);
+    r.tape = tmp.get<uint64_t>(tp_cap);
+    uint64_t *d_sum = tmp.get<uint64_t>(8);
+    if (STREAM) {
+        r.doc_first = tmp.get<uint32_t>(n + 1);
+        r.doc_tape = tmp.get<uint64_t>(n + 1);
+        r.doc_status = tmp.get<uint64_t>(n);
     }
-    uint32_t total;
-    uint32_t run = (uint32_t)block_before[blockIdx.x] + scan32_block_exclusive(mine, s_w, total);
-#pragma unroll
-    for (int j = 0; j < SCAN_PER_THREAD; j++) {
-        if (k0 + j < n) x[k0 + j] = run;
-        run += v[j];
-    }
-}
-// exclusive scan of x[0 .. n) in place on stream s; *d_total (device) receives the grand total
-cudaError_t scan32_exclusive(uint32_t *x, uint64_t n, unsigned long long *d_total, cudaMemPool_t pool, cudaStream_t s) {
-    const uint64_t nblocks = (n + SCAN_BLOCK - 1) / SCAN_BLOCK;
-    uint64_t *d_totals = nullptr;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_totals, nblocks * 8, pool, s);
-    if (e != cudaSuccess) return e;
-    scan32_totals_kernel<<<(unsigned)nblocks, SCAN_THREADS, 0, s>>>(x, n, d_totals);
-    scan_of_totals_kernel<<<1, 1024, 0, s>>>(d_totals, (uint32_t)nblocks, d_total);
-    scan32_apply_kernel<<<(unsigned)nblocks, SCAN_THREADS, 0, s>>>(x, n, d_totals);
-    e = cudaGetLastError();
-    cudaFreeAsync(d_totals, s);
-    return e;
+    if (tmp.failed) return SJB200_MEMALLOC;
+    int32_t rc = sjb200_stage2_primitives_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, r.strbuf, sb_cap, d_sum);
+    if (rc != SJB200_SUCCESS) return rc;
+    if constexpr (STREAM)
+        rc = sjb200_stage2_stream_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, r.tape, tp_cap, r.doc_first, r.doc_tape, r.doc_status,
+                                               d_sum + 4);
+    else
+        rc = sjb200_stage2_tape_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, r.tape, tp_cap, d_sum + 4);
+    if (rc != SJB200_SUCCESS) return rc;
+    CK(cudaMemcpyAsync(&r.sum, d_sum, sizeof r.sum, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return SJB200_SUCCESS;
 }
 
 }  // namespace
@@ -632,65 +692,11 @@ int32_t sjb200_stage2_tape_device_async(sjb200_ctx *c, const uint8_t *d_buf, uin
     if (len > 0xFFFFFFFFull || n > 0x7FFFFFF0ull) return SJB200_CAPACITY;   // tape positions are 32 bit: 2 n + 2 words must fit
     if (n == 0) return SJB200_EMPTY;   // json_iterator.mojo:45-46 (at_eof)
     CK(cudaSetDevice(c->device));
-    cudaStream_t s = c->stream;
-    unsigned long long *summary = reinterpret_cast<unsigned long long *>(d_summary);
     // summary: [0] first error as (index << 16 | rank of the check at that token << 8 | code), all ones = SUCCESS; [1] tape words of the tokens; [2] tape length; [3] inexact doubles
-    CK(cudaMemsetAsync(d_summary, 0xFF, 8, s));
-    CK(cudaMemsetAsync(d_summary + 1, 0, 24, s));
-    const uint64_t nblk = (n + TAPE_BLOCK - 1) / TAPE_BLOCK;
-    const uint32_t ntiles = (uint32_t)((n + MS_TILE - 1) / MS_TILE);
-    const size_t hist_entries = (size_t)2 * MS_CLASSES * ntiles;
-    Stk *d_stk = nullptr;
-    uint32_t *d_words = nullptr, *d_slot = nullptr, *d_rank = nullptr, *d_sorted = nullptr, *d_hist = nullptr;
-    uint8_t *d_cls = nullptr;
-    unsigned long long *d_tot = nullptr;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_stk, nblk * sizeof(Stk), c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_words, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_cls, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_slot, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_rank, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sorted, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_hist, hist_entries * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tot, 32, c->pool, s);
-    auto release = [&]() {
-        if (d_stk) cudaFreeAsync(d_stk, s);
-        if (d_words) cudaFreeAsync(d_words, s);
-        if (d_cls) cudaFreeAsync(d_cls, s);
-        if (d_slot) cudaFreeAsync(d_slot, s);
-        if (d_rank) cudaFreeAsync(d_rank, s);
-        if (d_sorted) cudaFreeAsync(d_sorted, s);
-        if (d_hist) cudaFreeAsync(d_hist, s);
-        if (d_tot) cudaFreeAsync(d_tot, s);
-    };
-    if (e != cudaSuccess) {
-        release();
-        cudaGetLastError();
-        return SJB200_MEMALLOC;
-    }
-    // depth / container type: the bit-stack scan; then the grammar, the words and the multisplit classes
-    tape_stack_totals_kernel<false><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_stk, nullptr);
-    tape_stack_scan_kernel<false><<<1, 1024, 0, s>>>(d_stk, (uint32_t)nblk);
-    tape_grammar_kernel<false><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_stk, d_words, d_cls, summary, StreamArgs{});
-    // where every token's words go
-    e = scan32_exclusive(d_words, n, summary + 1, c->pool, s);
-    // brackets and commas by depth: two class-major histograms, each scanned on its own, then the ranks
-    if (e == cudaSuccess) {
-        tape_multisplit_hist_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist);
-        e = scan32_exclusive(d_hist, (uint64_t)MS_CLASSES * ntiles, d_tot, c->pool, s);                                     // B: total = number of brackets
-    }
-    if (e == cudaSuccess) e = scan32_exclusive(d_hist + (size_t)MS_CLASSES * ntiles, (uint64_t)MS_CLASSES * ntiles, d_tot + 1, c->pool, s);   // A
-    uint32_t nbrackets_upper = (uint32_t)(n < 0xFFFFFFFFull ? n : 0xFFFFFFFFull);
-    if (e == cudaSuccess) {
-        tape_multisplit_rank_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist, 0u, d_slot, d_rank, d_sorted);
-        const unsigned grid = (unsigned)((n + 255) / 256 < (uint64_t)c->sm_count * 32 ? (n + 255) / 256 : (uint64_t)c->sm_count * 32);
-        tape_emit_kernel<false><<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_value, d_str_off, d_words, d_cls, d_slot, d_rank, d_sorted, nbrackets_upper,
-                                                     d_tape, tape_capacity, summary, StreamArgs{});
-        tape_roots_kernel<<<1, 1, 0, s>>>(d_tape, tape_capacity, summary + 1, summary);
-        e = cudaGetLastError();
-    }
-    release();
-    c->launches += 14;
-    return e == cudaSuccess ? SJB200_SUCCESS : cuda_err(e);
+    CK(cudaMemsetAsync(d_summary, 0xFF, 8, c->stream));
+    CK(cudaMemsetAsync(d_summary + 1, 0, 24, c->stream));
+    return stage2_walk<false>(c, d_buf, len, d_idx, n, d_kind, d_err, d_value, d_str_off, d_tape, tape_capacity,
+                              reinterpret_cast<unsigned long long *>(d_summary), nullptr, nullptr, nullptr);
 }
 
 // Stage 2 over a stream of documents (include/simdjson_b200.h): the same launches as the single-document walk, on the
@@ -705,88 +711,12 @@ int32_t sjb200_stage2_stream_device_async(sjb200_ctx *c, const uint8_t *d_buf, u
     if (len > 0xFFFFFFFFull || n >= (1ull << 30)) return SJB200_CAPACITY;   // tape positions are 32 bit: up to 4 n words
     if (n == 0) return SJB200_EMPTY;
     CK(cudaSetDevice(c->device));
-    cudaStream_t s = c->stream;
-    unsigned long long *summary = reinterpret_cast<unsigned long long *>(d_summary);
-    unsigned long long *doc_status = reinterpret_cast<unsigned long long *>(d_doc_status);
     // summary: [0] documents, [1] failing documents, [2] tape length, [3] inexact doubles
-    CK(cudaMemsetAsync(d_summary, 0, 32, s));
-    CK(cudaMemsetAsync(d_doc_status, 0xFF, n * 8, s));
-    const uint64_t nblk = (n + TAPE_BLOCK - 1) / TAPE_BLOCK;
-    const uint64_t dblk = (n + DEPTH_BLOCK - 1) / DEPTH_BLOCK;
-    const uint32_t ntiles = (uint32_t)((n + MS_TILE - 1) / MS_TILE);
-    const size_t hist_entries = (size_t)2 * MS_CLASSES * ntiles;
-    Stk *d_stk = nullptr;
-    uint32_t *d_words = nullptr, *d_slot = nullptr, *d_rank = nullptr, *d_sorted = nullptr, *d_hist = nullptr, *d_doc = nullptr;
-    uint8_t *d_cls = nullptr, *d_bytes = nullptr, *d_starts = nullptr;
-    int32_t *d_depth = nullptr;
-    unsigned long long *d_tot = nullptr;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_stk, nblk * sizeof(Stk), c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_words, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_cls, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_slot, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_rank, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sorted, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_hist, hist_entries * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tot, 32, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_doc, n * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_bytes, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_starts, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_depth, dblk * 4, c->pool, s);
-    auto release = [&]() {
-        if (d_stk) cudaFreeAsync(d_stk, s);
-        if (d_words) cudaFreeAsync(d_words, s);
-        if (d_cls) cudaFreeAsync(d_cls, s);
-        if (d_slot) cudaFreeAsync(d_slot, s);
-        if (d_rank) cudaFreeAsync(d_rank, s);
-        if (d_sorted) cudaFreeAsync(d_sorted, s);
-        if (d_hist) cudaFreeAsync(d_hist, s);
-        if (d_tot) cudaFreeAsync(d_tot, s);
-        if (d_doc) cudaFreeAsync(d_doc, s);
-        if (d_bytes) cudaFreeAsync(d_bytes, s);
-        if (d_starts) cudaFreeAsync(d_starts, s);
-        if (d_depth) cudaFreeAsync(d_depth, s);
-    };
-    if (e != cudaSuccess) {
-        release();
-        cudaGetLastError();
-        return SJB200_MEMALLOC;
-    }
-    const unsigned grid = (unsigned)((n + 255) / 256 < (uint64_t)c->sm_count * 32 ? (n + 255) / 256 : (uint64_t)c->sm_count * 32);
-    // where documents start: the bracket depth over the structural bytes
-    int32_t rc = sjb200_structural_bytes_device_async(c, d_buf, len, d_idx, n, d_bytes);
-    if (rc == SJB200_SUCCESS) rc = sjb200_document_starts_device_async(c, d_bytes, n, d_starts, d_depth, dblk);
-    if (rc != SJB200_SUCCESS) {
-        release();
-        return rc;
-    }
-    // the document of every token, and the first token of every document
-    stream_flags_kernel<<<grid, 256, 0, s>>>(d_starts, n, d_doc);
-    e = scan32_exclusive(d_doc, n, summary, c->pool, s);
-    if (e == cudaSuccess) stream_docs_kernel<<<grid, 256, 0, s>>>(d_starts, n, d_doc, d_doc_first, summary);
-    const StreamArgs sa{d_starts, d_doc, d_doc_first, d_doc_tape, doc_status};
-    // depth / container type inside each document: the segmented bit-stack scan; then the grammar, the words and the classes
-    if (e == cudaSuccess) {
-        tape_stack_totals_kernel<true><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_stk, d_starts);
-        tape_stack_scan_kernel<true><<<1, 1024, 0, s>>>(d_stk, (uint32_t)nblk);
-        tape_grammar_kernel<true><<<(unsigned)nblk, TAPE_THREADS, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_err, d_stk, d_words, d_cls, nullptr, sa);
-        e = scan32_exclusive(d_words, n, d_tot + 2, c->pool, s);
-    }
-    if (e == cudaSuccess) {
-        stream_roots_kernel<<<grid, 256, 0, s>>>(d_doc_first, d_words, n, summary, d_tot + 2, d_doc_tape, d_tape, tape_capacity, summary);
-        tape_multisplit_hist_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist);
-        e = scan32_exclusive(d_hist, (uint64_t)MS_CLASSES * ntiles, d_tot, c->pool, s);
-    }
-    if (e == cudaSuccess) e = scan32_exclusive(d_hist + (size_t)MS_CLASSES * ntiles, (uint64_t)MS_CLASSES * ntiles, d_tot + 1, c->pool, s);
-    if (e == cudaSuccess) {
-        tape_multisplit_rank_kernel<<<ntiles, 32, 0, s>>>(d_cls, n, ntiles, d_hist, 0u, d_slot, d_rank, d_sorted);
-        tape_emit_kernel<true><<<grid, 256, 0, s>>>(d_buf, len, d_idx, n, d_kind, d_value, d_str_off, d_words, d_cls, d_slot, d_rank, d_sorted, (uint32_t)n, d_tape,
-                                                    tape_capacity, summary, sa);
-        stream_failed_kernel<<<grid, 256, 0, s>>>(doc_status, summary);
-        e = cudaGetLastError();
-    }
-    release();
-    c->launches += 22;   // and 4 in the document split
-    return e == cudaSuccess ? SJB200_SUCCESS : cuda_err(e);
+    CK(cudaMemsetAsync(d_summary, 0, 32, c->stream));
+    CK(cudaMemsetAsync(d_doc_status, 0xFF, n * 8, c->stream));
+    return stage2_walk<true>(c, d_buf, len, d_idx, n, d_kind, d_err, d_value, d_str_off, d_tape, tape_capacity,
+                             reinterpret_cast<unsigned long long *>(d_summary), d_doc_first, d_doc_tape,
+                             reinterpret_cast<unsigned long long *>(d_doc_status));
 }
 
 // Host-to-host stage 2 over a stream of documents: sjb200_stage2's counterpart for NDJSON and concatenated JSON.
@@ -794,71 +724,25 @@ int32_t sjb200_stage2_stream(sjb200_ctx *c, uint64_t *tape_out, uint64_t tape_ca
                              uint64_t *doc_tape, uint64_t *doc_status, uint64_t max_docs, uint64_t *n_docs, uint64_t *n_failed, uint64_t *tape_len,
                              uint64_t *strbuf_len, uint64_t *inexact_doubles) {
     if (!c || !tape_out || !strbuf_out || !doc_first || !doc_tape || !doc_status) return SJB200_UNINITIALIZED;
-    if (c->resident_len == 0 || c->resident_n == 0) return SJB200_UNINITIALIZED;   // no successful stage 1 before this call
-    const uint64_t len = c->resident_len, n = c->resident_n;
-    CK(cudaSetDevice(c->device));
+    PoolBuffers tmp(c);
+    ResidentStage2 r;
+    const int32_t rc = stage2_resident<true>(c, tmp, r);
+    if (rc != SJB200_SUCCESS) return rc;
+    const uint64_t nd = r.sum.n_docs, tl = r.sum.tape_len, sb = r.sum.strbuf_len;
+    if (n_docs) *n_docs = nd;
+    if (n_failed) *n_failed = r.sum.n_failed;
+    if (tape_len) *tape_len = tl;
+    if (strbuf_len) *strbuf_len = sb;
+    if (inexact_doubles) *inexact_doubles = r.sum.inexact_doubles;
+    if (nd > max_docs || tl > tape_capacity || sb > strbuf_capacity) return SJB200_CAPACITY;
     cudaStream_t s = c->stream;
-    const uint64_t sb_cap = len + 2 * n + 64, tp_cap = 4 * n;
-    uint8_t *d_kind = nullptr, *d_err = nullptr, *d_sb = nullptr;
-    int64_t *d_val = nullptr;
-    uint64_t *d_off = nullptr, *d_tape = nullptr, *d_sum = nullptr, *d_dtape = nullptr, *d_dstatus = nullptr;
-    uint32_t *d_dfirst = nullptr;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_kind, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_err, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_val, n * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_off, n * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sb, sb_cap, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tape, tp_cap * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sum, 64, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dfirst, (n + 1) * 4, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dtape, (n + 1) * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_dstatus, n * 8, c->pool, s);
-    auto release = [&]() {
-        if (d_kind) cudaFreeAsync(d_kind, s);
-        if (d_err) cudaFreeAsync(d_err, s);
-        if (d_val) cudaFreeAsync(d_val, s);
-        if (d_off) cudaFreeAsync(d_off, s);
-        if (d_sb) cudaFreeAsync(d_sb, s);
-        if (d_tape) cudaFreeAsync(d_tape, s);
-        if (d_sum) cudaFreeAsync(d_sum, s);
-        if (d_dfirst) cudaFreeAsync(d_dfirst, s);
-        if (d_dtape) cudaFreeAsync(d_dtape, s);
-        if (d_dstatus) cudaFreeAsync(d_dstatus, s);
-    };
-    if (e != cudaSuccess) {
-        release();
-        cudaGetLastError();
-        return SJB200_MEMALLOC;
-    }
-    int32_t rc = sjb200_stage2_primitives_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_sb, sb_cap, d_sum);
-    if (rc == SJB200_SUCCESS)
-        rc = sjb200_stage2_stream_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_tape, tp_cap, d_dfirst, d_dtape, d_dstatus, d_sum + 4);
-    uint64_t sum[8] = {};
-    if (rc == SJB200_SUCCESS) {
-        e = cudaMemcpyAsync(sum, d_sum, 64, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) rc = cuda_err(e);
-    }
-    if (rc == SJB200_SUCCESS) {
-        const uint64_t sb = sum[1], nd = sum[4], tl = sum[6];
-        if (n_docs) *n_docs = nd;
-        if (n_failed) *n_failed = sum[5];
-        if (tape_len) *tape_len = tl;
-        if (strbuf_len) *strbuf_len = sb;
-        if (inexact_doubles) *inexact_doubles = sum[7];
-        if (nd > max_docs || tl > tape_capacity || sb > strbuf_capacity) rc = SJB200_CAPACITY;
-        if (rc == SJB200_SUCCESS) {
-            e = cudaMemcpyAsync(tape_out, d_tape, tl * 8, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess && sb) e = cudaMemcpyAsync(strbuf_out, d_sb, sb, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(doc_first, d_dfirst, (nd + 1) * 4, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(doc_tape, d_dtape, (nd + 1) * 8, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(doc_status, d_dstatus, nd * 8, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e != cudaSuccess) rc = cuda_err(e);
-        }
-    }
-    release();
-    return rc;
+    CK(cudaMemcpyAsync(tape_out, r.tape, tl * 8, cudaMemcpyDeviceToHost, s));
+    if (sb) CK(cudaMemcpyAsync(strbuf_out, r.strbuf, sb, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(doc_first, r.doc_first, (nd + 1) * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(doc_tape, r.doc_tape, (nd + 1) * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(doc_status, r.doc_status, nd * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return SJB200_SUCCESS;
 }
 
 // Host-to-host stage 2, the drop-in for DomParserImplementation.stage2 (include/generic/dom_parser_implementation.mojo:71-83):
@@ -867,59 +751,22 @@ int32_t sjb200_stage2_stream(sjb200_ctx *c, uint64_t *tape_out, uint64_t tape_ca
 int32_t sjb200_stage2(sjb200_ctx *c, uint64_t *tape_out, uint64_t tape_capacity, uint8_t *strbuf_out, uint64_t strbuf_capacity, uint64_t *tape_len,
                       uint64_t *strbuf_len, uint64_t *inexact_doubles) {
     if (!c || !tape_out || !strbuf_out) return SJB200_UNINITIALIZED;
-    if (c->resident_len == 0 || c->resident_n == 0) return SJB200_UNINITIALIZED;   // no successful stage 1 before this call
-    const uint64_t len = c->resident_len, n = c->resident_n;
-    CK(cudaSetDevice(c->device));
+    PoolBuffers tmp(c);
+    ResidentStage2 r;
+    int32_t rc = stage2_resident<false>(c, tmp, r);
+    if (rc != SJB200_SUCCESS) return rc;
+    const uint64_t tl = r.sum.tape_len, sb = r.sum.strbuf_len;
+    if (tape_len) *tape_len = tl;
+    if (strbuf_len) *strbuf_len = sb;
+    if (inexact_doubles) *inexact_doubles = r.sum.inexact_doubles;
+    rc = r.sum.verdict == ~0ull ? SJB200_SUCCESS : (int32_t)(r.sum.verdict & 0xFF);
+    if (rc == SJB200_SUCCESS && (tl > tape_capacity || sb > strbuf_capacity)) rc = SJB200_CAPACITY;
+    if (rc != SJB200_SUCCESS) return rc;
     cudaStream_t s = c->stream;
-    const uint64_t sb_cap = len + 2 * n + 64, tp_cap = 2 * n + 2;
-    uint8_t *d_kind = nullptr, *d_err = nullptr, *d_sb = nullptr;
-    int64_t *d_val = nullptr;
-    uint64_t *d_off = nullptr, *d_tape = nullptr, *d_sum = nullptr;
-    cudaError_t e = cudaMallocFromPoolAsync(&d_kind, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_err, n, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_val, n * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_off, n * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sb, sb_cap, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_tape, tp_cap * 8, c->pool, s);
-    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_sum, 64, c->pool, s);
-    auto release = [&]() {
-        if (d_kind) cudaFreeAsync(d_kind, s);
-        if (d_err) cudaFreeAsync(d_err, s);
-        if (d_val) cudaFreeAsync(d_val, s);
-        if (d_off) cudaFreeAsync(d_off, s);
-        if (d_sb) cudaFreeAsync(d_sb, s);
-        if (d_tape) cudaFreeAsync(d_tape, s);
-        if (d_sum) cudaFreeAsync(d_sum, s);
-    };
-    if (e != cudaSuccess) {
-        release();
-        cudaGetLastError();
-        return SJB200_MEMALLOC;
-    }
-    int32_t rc = sjb200_stage2_primitives_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_sb, sb_cap, d_sum);
-    if (rc == SJB200_SUCCESS) rc = sjb200_stage2_tape_device_async(c, c->d_in, len, c->d_out, n, d_kind, d_err, d_val, d_off, d_tape, tp_cap, d_sum + 4);
-    uint64_t sum[8] = {};
-    if (rc == SJB200_SUCCESS) {
-        e = cudaMemcpyAsync(sum, d_sum, 64, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) rc = cuda_err(e);
-    }
-    if (rc == SJB200_SUCCESS) {
-        const uint64_t sb = sum[1], tl = sum[6];
-        if (tape_len) *tape_len = tl;
-        if (strbuf_len) *strbuf_len = sb;
-        if (inexact_doubles) *inexact_doubles = sum[7];
-        rc = sum[4] == ~0ull ? SJB200_SUCCESS : (int32_t)(sum[4] & 0xFF);
-        if (rc == SJB200_SUCCESS && (tl > tape_capacity || sb > strbuf_capacity)) rc = SJB200_CAPACITY;
-        if (rc == SJB200_SUCCESS) {
-            e = cudaMemcpyAsync(tape_out, d_tape, tl * 8, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess && sb) e = cudaMemcpyAsync(strbuf_out, d_sb, sb, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e != cudaSuccess) rc = cuda_err(e);
-        }
-    }
-    release();
-    return rc;
+    CK(cudaMemcpyAsync(tape_out, r.tape, tl * 8, cudaMemcpyDeviceToHost, s));
+    if (sb) CK(cudaMemcpyAsync(strbuf_out, r.strbuf, sb, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return SJB200_SUCCESS;
 }
 
 }  // extern "C"

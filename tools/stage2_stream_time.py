@@ -3,8 +3,9 @@
   (a) primitives + stream walk (sjb200_stage2_stream_device_async) on synth.ndjson of --mib MiB
   (b) primitives + single-document walk (sjb200_stage2_tape_device_async) on synth.status_array of --mib MiB
   (c) (b) with another build of the library (--other-lib, e.g. one built from the parent commit), in the same process
+  (d) (a) with that other build
 
-Stage 1 runs once per input, untimed; the inputs and outputs stay on the device.  The runs of (a), (b) and (c) alternate
+Stage 1 runs once per input, untimed; the inputs and outputs stay on the device.  The runs of (a) to (d) alternate
 within every repetition, after --warmup untimed rounds of each.  Prints the card, its power limit and one line per
 measurement: median and spread in ms, and tokens per second."""
 import argparse
@@ -85,7 +86,9 @@ def main():
     this = bind(_native.LIB_PATH)
     runs = [("a stream walk, ndjson", stream, this, "ndjson"), ("b single walk, status_array", single, this, "status_array")]
     if args.other_lib:
-        runs.append(("c single walk, status_array, other build", single, bind(args.other_lib), "status_array"))
+        other = bind(args.other_lib)
+        runs.append(("c single walk, status_array, other build", single, other, "status_array"))
+        runs.append(("d stream walk, ndjson, other build", stream, other, "ndjson"))
     times = {r[0]: [] for r in runs}
     for rep in range(args.warmup + args.reps):
         for label, fn, (L, ctx), _ in runs:
