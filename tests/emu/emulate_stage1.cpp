@@ -542,6 +542,307 @@ extern "C" int32_t emu_stage1_stream(const uint8_t *buf, uint64_t len, uint32_t 
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// The stream pipeline with its UTF-8 deferral as the classify kernel does it (csrc/stage1_stream.cuh,
+// stage1_stream_classify_kernel, and warp_compute<UTF8, 1> in csrc/stage1_kernel.cuh):
+//   - per chunk, the flagged lanes (any_hi: a byte >= 0x80 in the lane or in the 4 bytes before it).  More than
+//     U8_DEFER_MAX = 8: the chunk validates inline, the carry from the previous lane computed only if some lane of the
+//     chunk passes the straddle gate; 1 to 8: the k-th flagged lane parks {bit planes, prev, end bit} in slot k of the
+//     warp's ring.
+//   - the schedule: `warps` warps in the grid; warp g first takes chunks 4g .. 4g+3, the runs after the first 4 * warps
+//     chunks go to warps in the order a seeded generator picks them (any order the ticket counter can produce); a warp
+//     works through its runs in the order it drew them.
+//   - one 32-slot ring per warp, kept across its runs, validated when a chunk leaves more than 32 - 8 slots in use
+//     (mid-run flush) and when the warp runs out of chunks (end-of-warp flush).
+//   - the fold of a violation among parked lanes (stage1_persistent.cuh): utf8_error = 1, and UTF8_ERROR only if the
+//     verdict is SUCCESS and flag 1 is set.
+// Besides the results of emu_stage1_stream it reports the flushes (stats[0] mid-run, stats[1] end-of-warp, stats[2]
+// the largest fill of a ring at a flush, stats[3] the mask of the slots any lane was parked in, stats[4] the chunks
+// validated inline) and, for each document byte position probe_pos[i], how the lane holding it was validated:
+// probe_out[4 i ..] = {kind (0 no byte >= 0x80 anywhere near: skipped, 1 inline, 2 parked), warp, slot, flush kind
+// (1 mid-run, 2 end-of-warp)}, -1 where not applicable.
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+constexpr int DEFER_MAX = 8, RING = 32, RUN = 4;
+
+struct Parked {
+    uint32_t pl[8], ph[8], prev, ends;
+    int64_t chunk;
+    int lane;
+};
+
+bool parked_lane_bad(const Parked &s) {   // validate_parked_lanes, one lane
+    Utf8Pre32 ul, uh;
+    utf8_pre32(s.pl, ul);
+    utf8_pre32(s.ph, uh);
+    const Utf8Carry uc = utf8_carry_from_prev_word(s.prev);
+    uint32_t tail_must;
+    const uint64_t ue = utf8_errors64(ul, uh, uc, &tail_must);
+    return (ue != 0) || (s.ends != 0 && tail_must != 0);
+}
+
+bool straddle_gate(uint32_t prev) { return (prev & (prev << 1) & 0x80808000u) != 0; }   // stage1_kernel.cuh, inline path
+
+uint64_t splitmix(uint64_t &s) {
+    uint64_t z = (s += 0x9E3779B97F4A7C15ull);
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+}  // namespace
+
+extern "C" int32_t emu_stage1_stream_sched(const uint8_t *buf, uint64_t len, uint32_t mis, uint32_t *out, uint64_t cap, uint32_t *n_out,
+                                           uint64_t *n_written_out, int32_t *utf8_err_out, int32_t *spec_out, uint32_t flags,
+                                           uint32_t warps, uint64_t seed, int64_t *stats, const uint64_t *probe_pos, uint32_t nprobe,
+                                           int32_t *probe_out) {
+    for (int k = 0; k < 5; k++) stats[k] = 0;
+    for (uint32_t i = 0; i < 4 * nprobe; i++) probe_out[i] = -1;
+    if (spec_out) *spec_out = 0;
+    if (len == 0 || warps == 0) return 13;
+    const int64_t alen = (int64_t)mis + (int64_t)len;
+    const int64_t nchunks = (alen + 2047) / 2048;
+    std::vector<uint8_t> mem((size_t)(nchunks * 2048 + 64));
+    for (size_t i = 0; i < mem.size(); i++) mem[i] = (i & 1) ? 0x5C : 0xF4;  // hostile bytes around the document
+    memcpy(mem.data() + mis, buf, (size_t)len);
+    const int64_t last = nchunks - 1;
+    const int64_t last_bytes = alen - last * 2048;
+
+    // ---- classify: everything but the parked lanes' validation, per chunk in any order ----
+    std::vector<uint64_t> plane0((size_t)nchunks * 32), plane1((size_t)nchunks * 32);
+    std::vector<Summary> sum((size_t)nchunks);
+    std::vector<std::vector<Parked>> parks((size_t)nchunks);   // the chunk's parked lanes in slot order
+    std::vector<uint8_t> kind((size_t)nchunks * 32, 0);        // per lane: 0 skipped, 1 inline, 2 parked
+    std::vector<uint8_t> stage(32 + 2048);
+    bool gave_up = false;
+    for (int64_t c = 0; c < nchunks; c++) {
+        for (size_t i = 0; i < stage.size(); i++) stage[i] = 0x5C;
+        const int64_t nb = c == last ? ((last_bytes + 15) & ~15ll) : 2048;
+        memcpy(stage.data() + 32, mem.data() + c * 2048, (size_t)nb);
+        if (c > 0) memcpy(stage.data(), mem.data() + c * 2048 - 32, 32);
+        const uint8_t *chunk = stage.data() + 32;
+        const bool edge = (c == 0) || (c == last && last_bytes < 2048);
+        PrevState wst = {0, 0, 0};
+        if (c > 0) {
+            uint32_t bsm = 0;
+            for (int l = 0; l < 32; l++) bsm |= (uint32_t)(chunk[-1 - l] == 0x5C) << l;
+            wst = prev_state(bsm, 32, chunk[-1]);
+        }
+        if (wst.unresolved) gave_up = true;
+        LaneMasks m[32];
+        uint32_t pl[32][8], ph[32][8], prev[32], ends[32], hi_lanes = 0, gate = 0, A = 0, O = 0;
+        for (int l = 0; l < 32; l++) {
+            const int64_t g0 = c * 2048 + (int64_t)l * 64;
+            uint32_t words[16];
+            memcpy(words, chunk + l * 64, 64);
+            memcpy(&prev[l], chunk + l * 64 - 4, 4);
+            ends[l] = (c == last) && ((int64_t)l * 64 + 64 == last_bytes);
+            if (edge) {
+                for (int k = 0; k < 16; k++) words[k] = mask_word(words[k], g0 + 4 * k, mis, alen);
+                prev[l] = (g0 == 0) ? 0x20202020u : mask_word(prev[l], g0 - 4, mis, alen);
+            }
+            bitplanes32(words, pl[l]);
+            bitplanes32(words + 8, ph[l]);
+            Classes32 cl, ch;
+            classify_json32(pl[l], cl);
+            classify_json32(ph[l], ch);
+            m[l].bs = join64(cl.bs, ch.bs);
+            m[l].rq = join64(cl.rq, ch.rq);
+            m[l].op = join64(cl.op, ch.op);
+            m[l].ws = join64(cl.ws, ch.ws);
+            m[l].ctl = join64(cl.ctl, ch.ctl);
+            hi_lanes |= (uint32_t)(((pl[l][7] | ph[l][7]) != 0) || ((prev[l] & 0x80808080u) != 0)) << l;
+            gate |= (uint32_t)straddle_gate(prev[l]) << l;
+            A |= (uint32_t)lane_all_backslash(m[l].bs) << l;
+            O |= lane_trailing_run_parity(m[l].bs) << l;
+        }
+        uint32_t u8err = 0;
+        if (popc32(hi_lanes) <= DEFER_MAX) {
+            for (int l = 0; l < 32; l++) {
+                if (!((hi_lanes >> l) & 1u)) continue;
+                Parked s;
+                memcpy(s.pl, pl[l], sizeof s.pl);
+                memcpy(s.ph, ph[l], sizeof s.ph);
+                s.prev = prev[l];
+                s.ends = ends[l];
+                s.chunk = c;
+                s.lane = l;
+                parks[(size_t)c].push_back(s);
+                kind[(size_t)c * 32 + l] = 2;
+            }
+        } else {
+            stats[4]++;
+            for (int l = 0; l < 32; l++) {
+                kind[(size_t)c * 32 + l] = 1;
+                Utf8Pre32 ul, uh;
+                utf8_pre32(pl[l], ul);
+                utf8_pre32(ph[l], uh);
+                Utf8Carry uc = {0, 0, 0, 0};
+                if (gate) uc = utf8_carry_from_prev_word(prev[l]);
+                uint32_t tail_must;
+                const uint64_t ue = utf8_errors64(ul, uh, uc, &tail_must);
+                u8err |= (ue != 0) || (ends[l] && tail_must != 0);
+            }
+        }
+        uint32_t PB = 0, NQ = 0;
+        LaneQuotes q[32];
+        for (int l = 0; l < 32; l++) {
+            q[l] = lane_quotes(m[l], warp_lane_e_in(A, O, l, wst.e));
+            PB |= (uint32_t)(q[l].ps >> 63) << l;
+            NQ |= (uint32_t)(q[l].nqs >> 63) << l;
+        }
+        uint32_t fl = 0, wc0 = 0, wc1 = 0;
+        for (int l = 0; l < 32; l++) {
+            const uint32_t rel = (uint32_t)popc32(PB & ((1u << l) - 1u)) & 1u;
+            const uint32_t p_in = l ? ((NQ >> (l - 1)) & 1u) : wst.p;
+            const LaneDual d = lane_structurals_dual(m[l], q[l], rel, p_in);
+            plane0[(size_t)c * 32 + l] = d.m0;
+            plane1[(size_t)c * 32 + l] = d.m1;
+            wc0 += (uint32_t)popc64(d.m0);
+            wc1 += (uint32_t)popc64(d.m1);
+            fl |= (d.u0 << 1) | (d.u1 << 2);
+        }
+        sum[(size_t)c] = {wc0, wc1, fl | (u8err << 3) | ((uint32_t)popc32(PB) & 1u)};
+    }
+
+    // ---- the schedule: which warp takes which run, in which order ----
+    const int64_t nruns = (nchunks + RUN - 1) / RUN;
+    std::vector<std::vector<int64_t>> runs_of((size_t)warps);
+    for (int64_t r = 0; r < nruns && r < (int64_t)warps; r++) runs_of[(size_t)r].push_back(r);
+    uint64_t rng = seed;
+    for (int64_t r = warps; r < nruns; r++) runs_of[(size_t)(splitmix(rng) % warps)].push_back(r);
+
+    // ---- each warp's ring ----
+    std::vector<int32_t> slot_of((size_t)nchunks * 32, -1), warp_of((size_t)nchunks * 32, -1), flush_of((size_t)nchunks * 32, -1);
+    bool u8_bad = false;
+    std::vector<const Parked *> ring;
+    auto flush = [&](int how) {
+        stats[how == 1 ? 0 : 1]++;
+        if ((int64_t)ring.size() > stats[2]) stats[2] = (int64_t)ring.size();
+        for (const Parked *s : ring) {
+            flush_of[(size_t)s->chunk * 32 + s->lane] = how;
+            u8_bad |= parked_lane_bad(*s);
+        }
+        ring.clear();
+    };
+    for (uint32_t w = 0; w < warps; w++) {
+        ring.clear();
+        for (int64_t r : runs_of[w]) {
+            for (int64_t c = r * RUN; c < (r + 1) * RUN && c < nchunks; c++) {
+                for (const Parked &s : parks[(size_t)c]) {
+                    if (ring.size() >= (size_t)RING) return -110;   // cannot happen: a flush leaves room for 8
+                    slot_of[(size_t)c * 32 + s.lane] = (int32_t)ring.size();
+                    warp_of[(size_t)c * 32 + s.lane] = (int32_t)w;
+                    stats[3] |= 1ll << ring.size();
+                    ring.push_back(&s);
+                }
+                if (ring.size() > (size_t)(RING - DEFER_MAX)) flush(1);
+            }
+        }
+        if (!ring.empty()) flush(2);
+    }
+    for (uint32_t i = 0; i < nprobe; i++) {
+        const int64_t g = (int64_t)probe_pos[i] + mis;
+        if (probe_pos[i] >= len) continue;
+        const size_t j = (size_t)(g / 64);
+        probe_out[4 * i] = kind[j];
+        if (kind[j] == 2) {
+            probe_out[4 * i + 1] = warp_of[j];
+            probe_out[4 * i + 2] = slot_of[j];
+            probe_out[4 * i + 3] = flush_of[j];
+        }
+    }
+    if (gave_up) {
+        if (spec_out) *spec_out = 1;
+        return 0;
+    }
+
+    // ---- span scan and flatten, as emu_stage1_stream (the deferred lanes are not in the summaries) ----
+    const int64_t BLOCK = 4096, PER_THREAD = 4;
+    const int64_t nblocks = (nchunks + BLOCK - 1) / BLOCK;
+    std::vector<SpanAcc> block((size_t)nblocks);
+    for (int64_t b = 0; b < nblocks; b++) {
+        SpanAcc acc = span_empty();
+        for (int64_t c = b * BLOCK; c < nchunks && c < (b + 1) * BLOCK; c++) acc = span_concat(acc, span_of(sum[(size_t)c]));
+        block[(size_t)b] = acc;
+    }
+    std::vector<uint64_t> carry((size_t)nchunks);
+    TilePrefix fin = {0, 0, 0, 0, 0};
+    SpanAcc before = span_empty();
+    for (int64_t b = 0; b < nblocks; b++) {
+        SpanAcc run = before;
+        for (int64_t c0 = b * BLOCK; c0 < nchunks && c0 < (b + 1) * BLOCK; c0 += PER_THREAD) {
+            Summary s4[4] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
+            for (int k = 0; k < PER_THREAD; k++)
+                if (c0 + k < nchunks) s4[k] = sum[(size_t)(c0 + k)];
+            for (int k = 0; k < PER_THREAD; k++) run = span_concat(run, span_of(s4[k]));
+            uint32_t par = run.par & 1u, cnt = run.c[0];
+            if (c0 < nchunks && c0 + PER_THREAD >= nchunks) {
+                fin.s_out = par;
+                fin.err = (run.un[0] ? EF_UNESCAPED : 0u) | (run.u8 ? EF_UTF8 : 0u);
+                fin.count = cnt;
+            }
+            for (int k = PER_THREAD - 1; k >= 0; k--) {
+                const uint32_t s_in = (par ^ s4[k].flags) & 1u;
+                cnt -= s_in ? s4[k].c1 : s4[k].c0;
+                par = s_in;
+                if (c0 + k < nchunks) carry[(size_t)(c0 + k)] = (uint64_t)cnt | (s_in ? (1ull << 63) : 0ull);
+            }
+        }
+        before = span_concat(before, block[(size_t)b]);
+    }
+    for (int64_t c = 0; c < nchunks; c++) {
+        const uint64_t cw = carry[(size_t)c];
+        const bool inside = (cw >> 63) != 0;
+        uint64_t o = cw & ((1ull << 40) - 1);
+        for (int l = 0; l < 32; l++) {
+            uint64_t st = inside ? plane1[(size_t)c * 32 + l] : plane0[(size_t)c * 32 + l];
+            const uint32_t v0 = (uint32_t)c * 2048u + (uint32_t)l * 64u - mis;
+            while (st) {
+                const int bit = __builtin_ctzll(st);
+                st &= st - 1;
+                if (o < cap) out[o] = v0 + (uint32_t)bit;
+                o++;
+            }
+        }
+    }
+    // ---- write_verdict (stage1_kernel.cuh) ----
+    const uint64_t n = fin.count;
+    int32_t err, utf8 = (fin.err & EF_UTF8) ? 1 : 0;
+    if (n_written_out) *n_written_out = n;
+    if (fin.s_out) err = 15;
+    else if (fin.err & EF_UNESCAPED) err = 14;
+    else if (n + 3 > cap) err = 1;
+    else {
+        if (n_out) *n_out = (uint32_t)n;
+        out[n] = (uint32_t)len;
+        out[n + 1] = (uint32_t)len;
+        out[n + 2] = 0;
+        err = n == 0 ? 13 : ((flags & 1u) && utf8) ? 11 : 0;
+    }
+    // ---- the fold by the persistent kernel launched behind the pipeline (stage1_persistent.cuh) ----
+    if (u8_bad) {
+        utf8 = 1;
+        if ((flags & 1u) && err == 0) err = 11;
+    }
+    if (utf8_err_out) *utf8_err_out = utf8;
+    return err;
+}
+
+// the straddle gate against the carry it guards: over every value of the three bytes before a lane (the fourth, the
+// lowest, does not enter either), the number of values for which the gate is closed but the carry is not {0, 0, 0, 0}
+extern "C" uint64_t emu_straddle_gate_misses(uint64_t *closed_out) {
+    uint64_t miss = 0, closed = 0;
+    for (uint32_t v = 0; v < (1u << 24); v++) {
+        const uint32_t prev = (v << 8) | 0x41u;
+        if (straddle_gate(prev)) continue;
+        closed++;
+        const Utf8Carry c = utf8_carry_from_prev_word(prev);
+        miss += (c.must | c.u | c.v | c.w) != 0;
+    }
+    *closed_out = closed;
+    return miss;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // Balanced flatten of one unit (csrc/stage1_split.cuh: stage1_flatten2_kernel) on the host: 128 mask words in stream order
 // (lane t owns words 4t .. 4t+3), every lane extracts the same number q of consecutive indexes.  Same steps as the kernel:
 // entries {word bit-reversed, next non-empty entry}, prefix counts, the table "share u starts in lane t" filled by the word

@@ -737,7 +737,8 @@ def test_maximum_length_document(kernel):
 def test_utf8_verdicts_sparse_lanes(dev, scratch, kernel):
     """Valid and invalid UTF-8 sequences in otherwise ASCII documents, placed so that they straddle lane (64 B) and chunk
     (2 KiB) boundaries, sit at the very start / end of the document, or follow a lane that is pure ASCII: in the stream
-    pipeline these are exactly the lanes whose validation is deferred to stage1_utf8_lanes_kernel."""
+    pipeline these are lanes the classify kernel parks in its warp's ring and validates at a flush (validate_parked_lanes,
+    stage1_stream.cuh).  Every slot, both flushes and ticketed runs: tests/test_gpu_utf8_deferral.py."""
     seqs = list(cases.UTF8_VALID) + list(cases.UTF8_INVALID)
     for k, seq in enumerate(seqs):
         seq = seq if isinstance(seq, (bytes, bytearray)) else seq.encode("utf-8", "surrogatepass")
