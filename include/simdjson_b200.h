@@ -422,6 +422,36 @@ int32_t sjb200_stage2_stream_at_pointers(sjb200_ctx *ctx, const uint8_t *pointer
                                          uint8_t *type_out, uint8_t *code_out, int64_t *value_out, uint64_t cells_capacity, uint8_t *strbuf_out,
                                          uint64_t strbuf_capacity, uint64_t *n_docs, uint64_t *strbuf_len);
 
+/*
+ * String columns from pointer cells: the string cells of K columns of D cells (the type and value outputs of
+ * sjb200_at_pointers_device_async, [K][D], pointer-major) become K string columns in the offsets + bytes layout (Arrow,
+ * cuDF, torch nested tensors), on the device.
+ *
+ * Input: d_type and d_value (K x D cells each) and the string buffer the cells point into, strbuf_len bytes of it.  A cell
+ * with type '"' is a string: its bytes are those of the {uint32 length, bytes} record at d_strbuf + value.  Every other cell,
+ * found or not, contributes 0 bytes.
+ *
+ * Outputs:
+ *   d_offsets  K·D + 1 int64 (8-byte aligned): one exclusive prefix sum of the cell lengths over all K·D cells in cell order,
+ *              d_offsets[K·D] = total bytes.  Cell i's bytes are d_data[d_offsets[i] .. d_offsets[i + 1]); column k is
+ *              d_offsets[k·D .. k·D + D] inclusive (neighbouring columns share an endpoint), one contiguous slice of d_data.
+ *   d_data     every string's unescaped bytes exactly as its record holds them: no length words, no terminators.  Any
+ *              alignment.  Bytes at or past data_capacity are never written; every byte below min(total, data_capacity) is.
+ *              May be NULL: then only the offsets and the summary are written, so that a caller can size the buffer first.
+ *   d_summary  2 x uint64: [0] total bytes (the full figure, also when it exceeds data_capacity); [1] the number of string
+ *              cells whose record does not lie inside strbuf_len (the guard of the pointer lookups).  Those cells get length
+ *              0; cells sjb200_at_pointers_device_async wrote over the same buffer never trigger it.
+ * Every read stays inside d_type, d_value, d_offsets and strbuf_len, whatever the caller passes.
+ *
+ * UNINITIALIZED for a NULL ctx, d_offsets or d_summary, or, when K·D > 0, a NULL d_type, d_value or d_strbuf.  CAPACITY
+ * when K·D > 2^40.  K·D == 0: SUCCESS, d_offsets[0] = 0, summary zeroed.  Stream ordered on the context's stream, no host
+ * synchronisation; temporaries from its pool.  The copy is balanced by output bytes, not by cells: its cost does not
+ * depend on how the bytes are spread over the cells.
+ */
+int32_t sjb200_string_columns_device_async(sjb200_ctx *ctx, const uint8_t *d_type, const int64_t *d_value, uint64_t n_columns, uint64_t n_docs,
+                                           const uint8_t *d_strbuf, uint64_t strbuf_len, int64_t *d_offsets, uint8_t *d_data,
+                                           uint64_t data_capacity, uint64_t *d_summary);
+
 #ifdef __cplusplus
 }
 #endif

@@ -60,6 +60,7 @@ SIGNATURES = {
     "sjb200_stage2_stream": (_i32, [_vp, _vp, _u64, _vp, _u64, _vp, _vp, _vp, _u64, _pu64, _pu64, _pu64, _pu64, _pu64]),
     "sjb200_at_pointers_device_async": (_i32, [_vp, _vp, _u64, _vp, _u64, _vp, _vp, _u64, _vp, _pu64, _u64, _vp, _vp, _vp]),
     "sjb200_stage2_stream_at_pointers": (_i32, [_vp, _vp, _pu64, _u64, _vp, _vp, _vp, _u64, _vp, _u64, _pu64, _pu64]),
+    "sjb200_string_columns_device_async": (_i32, [_vp, _vp, _vp, _u64, _u64, _vp, _u64, _vp, _vp, _u64, _vp]),
 }
 
 _lib = None

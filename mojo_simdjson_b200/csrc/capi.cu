@@ -997,3 +997,4 @@ int32_t sjb200_batch_run_device(sjb200_ctx *c, const uint8_t *d_buf, const uint6
 #include "stage2_primitives.cuh"
 #include "stage2_tape.cuh"
 #include "stage2_pointer.cuh"
+#include "stage2_columns.cuh"

@@ -56,6 +56,29 @@ class PointerColumns:
         return t == ord("t"), (t == ord("t")) | (t == ord("f"))
 
 
+@dataclass
+class StringColumns:
+    """K string columns of D cells from Stage1Context.string_columns, in the offsets + bytes layout (include/simdjson_b200.h,
+    sjb200_string_columns_device_async): offsets (int64 [K·D + 1], one prefix sum over every cell, column k is
+    offsets[k·D .. k·D + D]), data (uint8 [total], the strings' bytes back to back), mask (bool [K, D], True for string
+    cells).  Every non-string cell is empty."""
+    offsets: torch.Tensor
+    data: torch.Tensor
+    mask: torch.Tensor
+    bounds: list[int]   # offsets[k·D] for k = 0 .. K, on the host: where each column's bytes start and end
+
+    def column(self, k: int) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """(offsets int64 [D + 1] rebased to 0, data uint8 view of the column's bytes, mask bool [D]) of column k."""
+        d = self.mask.shape[1]
+        return self.offsets[k * d : k * d + d + 1] - self.bounds[k], self.data[self.bounds[k] : self.bounds[k + 1]], self.mask[k]
+
+    def to_list(self, k: int) -> list:
+        """Column k on the host: bytes for string cells, None for every other cell."""
+        off, data, mask = (t.cpu() for t in self.column(k))
+        off, raw = off.tolist(), data.numpy().tobytes()
+        return [raw[off[d] : off[d + 1]] if m else None for d, m in enumerate(mask.tolist())]
+
+
 class Stage1Context:
     """One parser context per GPU; runs on torch's current stream of that device by default."""
 
@@ -258,6 +281,44 @@ class Stage1Context:
         if rc != errors.SUCCESS:
             raise RuntimeError(f"pointer lookup failed: {errors.NAMES.get(rc, rc)}")
         return cols
+
+    def string_columns(self, cols: PointerColumns, string_buf: torch.Tensor) -> StringColumns:
+        """The string cells of pointer columns as device string columns, offsets + bytes (include/simdjson_b200.h,
+        sjb200_string_columns_device_async).  `string_buf` is the buffer the cells point into.  The whole chain stays on the
+        device:
+
+            prims = ctx.stage2_primitives(buf, idx, n)
+            s = ctx.stage2_stream(buf, idx, n, prims)
+            cols = ctx.at_pointers(["/text", "/lang"], s["tape"], prims["string_buf"], s["doc_tape"], s["doc_status"])
+            strs = ctx.string_columns(cols, prims["string_buf"])
+            offsets, data, mask = strs.column(0)
+
+        Synchronises once to learn the total size: the offsets are computed first without the data, then the bytes are
+        gathered into a buffer of exactly that size.  Raises RuntimeError if a string cell's record lies outside
+        `string_buf` (cells at_pointers wrote over the same buffer never do)."""
+        assert string_buf.is_cuda and string_buf.dtype == torch.uint8 and string_buf.is_contiguous()
+        assert cols.type.is_contiguous() and cols.value.is_contiguous() and cols.type.shape == cols.value.shape
+        k, d = cols.type.shape
+        dev = cols.type.device
+        offsets = torch.empty(k * d + 1, dtype=torch.int64, device=dev)
+        summary = torch.empty(2, dtype=torch.int64, device=dev)
+
+        def call(data: torch.Tensor | None) -> None:
+            rc = self._lib.sjb200_string_columns_device_async(self._ctx, cols.type.data_ptr(), cols.value.data_ptr(), k, d, string_buf.data_ptr(),
+                                                              string_buf.numel(), offsets.data_ptr(), None if data is None else data.data_ptr(),
+                                                              0 if data is None else data.numel(), summary.data_ptr())
+            if rc != errors.SUCCESS:
+                raise RuntimeError(f"string columns failed: {errors.NAMES.get(rc, rc)}")
+
+        call(None)
+        total, bad = summary.tolist()
+        if bad:
+            raise RuntimeError(f"string columns: {bad} string cells point outside the string buffer")
+        bounds = offsets[::d].tolist() if d else [0] * (k + 1)
+        data = torch.empty(total, dtype=torch.uint8, device=dev)
+        if total:
+            call(data)
+        return StringColumns(offsets, data, cols.type == ord('"'), bounds)
 
     def last_elapsed_ms(self) -> float:
         return float(self._lib.sjb200_last_elapsed_ms(self._ctx))
